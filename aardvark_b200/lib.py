@@ -12,6 +12,7 @@ library is missing or no CUDA device is present, construction raises.
 """
 import ctypes as C
 import os
+import shutil
 import subprocess
 from typing import List, Sequence
 
@@ -41,7 +42,9 @@ def build(force=False, verbose=False):
     srcs.append(os.path.join(_HERE, "..", "include", "aardvark_b200.h"))
     if not force and os.path.exists(SO_PATH) and os.path.getmtime(SO_PATH) >= max(os.path.getmtime(s) for s in srcs):
         return SO_PATH
-    cmd = ["nvcc"] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", SO_PATH, srcs[0]]
+    # nvcc is often not on an ordinary user's PATH: fall back to the toolkit's usual locations
+    nvcc = shutil.which("nvcc") or os.path.join(os.environ.get("CUDA_HOME") or os.environ.get("CUDA_PATH") or "/usr/local/cuda", "bin", "nvcc")
+    cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", SO_PATH, srcs[0]]
     env = dict(os.environ)
     env.pop("CXX", None)
     env.pop("CC", None)

@@ -24,6 +24,9 @@ NVLink) brings the per-region / per-variant result arrays and the summary counte
          => e2e.seconds_per_genome (single call) is the "WGS compare wall-time" half of the metric
   --impl reference: the CPU restatement of the reference path (oracle "port"; the reference is Rust and cannot be
          built here) on the SAME whole batch, OpenMP over clusters on ALL host cores, whatever N is.
+
+  --dump-outputs DIR  after the timed steps, write what the last step returned to its caller as DIR/<name>.npy (see
+         dump_outputs); the workload is seeded, so two builds run with the same arguments can be compared array by array.
 """
 import argparse
 import json
@@ -132,6 +135,35 @@ def bin_h2d_bytes(batch, lo, hi):
     return (hi - lo) * 12 + ((hi - lo) * k + 1) * 8 + (v1 - v0) * 22 + pool
 
 
+DUMP_SAMPLE = 1 << 20        # indices kept per axis (regions, variants): the dump stays below 64 MB at any scale
+
+
+def dump_outputs(out_dir, arrays, n_regions, n_variants):
+    """Write a compare call's outputs as <out_dir>/<name>.npy.  `arrays`: name -> array over regions, over variants or
+    whole-batch (totals, block counts).  An axis longer than DUMP_SAMPLE keeps a fixed, seeded sample of its indices,
+    written as region_index / variant_index.  Small codes are stored as float32, edit distances, counters and indices as
+    float64 (both exact for the integers they hold)."""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = {}
+    for axis, n in (("region", n_regions), ("variant", n_variants)):
+        ix = np.arange(n) if n <= DUMP_SAMPLE else np.sort(np.random.default_rng(12345).choice(n, DUMP_SAMPLE, replace=False))
+        idx[axis] = ix
+        np.save(os.path.join(out_dir, f"{axis}_index.npy"), ix.astype(np.float64))
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        axis = "region" if name in ("status", "ed1", "ed2", "type_mask") else "variant" if name.startswith("var_") else None
+        if axis is not None:
+            a = a[:n_regions if axis == "region" else n_variants][idx[axis]]
+        dt = np.float32 if name in ("status", "type_mask", "totals_mask") or name.startswith("var_") else np.float64
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(dt))
+
+
+def compare_out_arrays(out):
+    """The arrays of a CompareOutputs (region_metrics=False) that bench.py dumps."""
+    return {f: getattr(out, f) for f in ("status", "ed1", "ed2", "type_mask", "var_expected", "var_observed", "var_class",
+                                         "totals", "totals_mask", "solved_blocks", "error_blocks")}
+
+
 def run_reference(args, rank):
     """--impl reference: the reference's CPU path (oracle port; the Rust crate cannot be built here) on the SAME whole
     batch the GPU arm solves, on all host cores (torchrun's OMP_NUM_THREADS=1 is overridden explicitly)."""
@@ -145,11 +177,13 @@ def run_reference(args, rank):
     cfg = abi.CompareCfg(50, 0, 0, 0)
     for _ in range(min(args.warmup, 1)):
         orc.compare_batch(batch, refs, cfg, n_threads=cores, region_metrics=False)
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
-        orc.compare_batch(batch, refs, cfg, n_threads=cores, region_metrics=False)
+        out = orc.compare_batch(batch, refs, cfg, n_threads=cores, region_metrics=False)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, compare_out_arrays(out), batch.n_regions, batch.n_variants)
     v = batch.n_regions * steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
@@ -157,7 +191,7 @@ def run_reference(args, rank):
         "vs_baseline": None, "dtype": "int32", "data": "synthetic",
         "config": {"workload": desc, "regions_per_step": batch.n_regions, "variants_per_step": batch.n_variants, "max_branch_factor": 50},
         "cpu_baseline": {"value": v, "unit": UNIT, "cores": cores, "kind": "port",
-                         "sample": f"the whole batch ({batch.n_regions} clusters) x {steps} steps (capped at 5), OpenMP dynamic over clusters, "
+                         "sample": f"the whole batch ({batch.n_regions} clusters) x {steps} steps, OpenMP dynamic over clusters, "
                                    "solve phase only; oracle built -O3 -march=native -flto on this host"},
         "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0, "seconds_per_genome": dt / steps},
         "gpu_launches": 0,
@@ -176,7 +210,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--in-flight", type=int, default=4,
                     help="passes in flight per GPU (one context + host thread each, avk_create_lane); 1 = one pass at a time")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, a seeded sample of "
+                         "regions and variants when there are more than 2^20 of either)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -363,6 +402,15 @@ def main():
             for f in OUT_FIELDS:       # this rank's bin of the gathered arrays == its own resident result
                 a, b = ((var_bins[0][0], var_bins[0][1]) if f.startswith("var_") else (lo, hi))
                 assert np.array_equal(merged[f][a:b], getattr(resident_out, f)[a:b]), f"gathered {f} differs from the resident result"
+    if args.dump_outputs and rank == 0:
+        # the last e2e step's results as its caller receives them (N > 1: the arrays gathered on rank 0)
+        if world == 1:
+            dumped = compare_out_arrays(out)
+        else:
+            dumped = {f: merged[f] for f in OUT_FIELDS}
+            dumped.update(totals=merged["totals"], totals_mask=np.array([merged["totals_mask"]]),
+                          solved_blocks=np.array([merged["solved"]]), error_blocks=np.array([merged["errors"]]))
+        dump_outputs(args.dump_outputs, dumped, batch.n_regions, batch.n_variants)
 
     # ---------------- aggregate over ranks: max time, summed bytes --------------------------------
     stats = torch.tensor([dev_ms, e2e_s * 1e3, pipe_ms, flight_ms if flight_ms is not None else dev_ms, e2e_single_s * 1e3],
