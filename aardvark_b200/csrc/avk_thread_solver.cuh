@@ -173,6 +173,7 @@ struct Solver {
     u32 f_X, f_Y, f_tp, f_Ef, f_failT, f_failQ, f_failF, f_other;
     int f_altT, f_altQ, f_side, f_alt_other;
     u32 f_mask;
+    bool f_mirror;                 // truth filter == query filter (mirror_lists): one pass per slot serves both sides
 
 #if defined(__CUDA_ARCH__)
     // on the device the workspaces sit side by side in dynamic shared memory: addressing them through the __shared__ array
@@ -707,6 +708,7 @@ struct Solver {
             // costs its alt_ed in both).  Counters accumulate in W.bp; nothing else is kept.
             case PC_F_BEGIN: {
                 for (int s = 0; s <= c.n_slots; ++s) for (int m = 0; m < 4; ++m) W.bp[s][m] = 0;
+                f_mirror = mirror_lists(W.res[best_r]);
                 h2 = 0;
                 pc = PC_F_HAP;
                 break;
@@ -763,6 +765,7 @@ struct Solver {
                 else if (nf == (f_side ? c.nQ : c.nT)) {                         // filtered == full haplotype
                     W.bp[1 + k][2 * f_side] += f_tp;
                     W.bp[1 + k][2 * f_side + 1] += f_side ? (2 * f_Y - f_tp + 2 * f_failQ) : (2 * f_X - f_tp + 2 * f_failT);
+                    if (f_mirror) { W.bp[1 + k][0] += f_tp; W.bp[1 + k][1] += 2 * f_Y - f_tp + 2 * f_failQ; }   // (X == Y, failT == failQ)
                     next = true;
                 } else {
                     SeqInfo fi;
@@ -777,7 +780,7 @@ struct Solver {
                     pc = PC_F_EF_DONE;
                     return;
                 }
-                if (next) { if (f_side == 1) f_side = 0; else { f_side = 1; k += 1; } }
+                if (next) { if (f_side == 1 && !f_mirror) f_side = 0; else { f_side = 1; k += 1; } }
                 break;
             }
             case PC_F_EF_DONE: {
@@ -798,7 +801,8 @@ struct Solver {
                 const u32 ftp = f_other + f_Ef - Zf;
                 W.bp[1 + k][2 * f_side] += ftp;
                 W.bp[1 + k][2 * f_side + 1] += 2 * f_Ef - ftp + 2 * f_failF;
-                if (f_side == 1) f_side = 0; else { f_side = 1; k += 1; }
+                if (f_mirror) { W.bp[1 + k][0] += ftp; W.bp[1 + k][1] += 2 * f_Ef - ftp + 2 * f_failF; }
+                if (f_side == 1 && !f_mirror) f_side = 0; else { f_side = 1; k += 1; }
                 pc = PC_F_SLOT;
                 break;
             }
@@ -808,6 +812,25 @@ struct Solver {
                 return;
             }
         }
+    }
+
+    // Basepair metrics of a result in which the truth and query lists are the same records (order t0 q0 t1 q1 ...: position,
+    // REF / ALT bytes, type slot) and each query record carries its ALT on exactly the haplotypes its truth twin does -- the
+    // usual true-positive cluster.  Then the two haplotypes of each side spell the same strings, and so does every per-type
+    // filter of them: ED(ref, truth filter) == ED(ref, query filter), ED(truth filter, query) == ED(truth, query filter)
+    // (edit distance is symmetric), X == Y and the skip sums agree, so the truth-filter pass of each slot (waffle_solver.rs
+    // :422-437) adds what the query-filter pass (:395-410) adds and is not run.
+    AVK_HD bool mirror_lists(const ResEnt &R) const {
+        const Work &W = w();
+        const int n = c.N;
+        if (c.nT != c.nQ || (n & 1)) return false;
+        for (int i = 0; i < n; i += 2) {
+            const VarInfo a = W.var[i], b = W.var[i + 1];
+            if (!is_truth(i) || is_truth(i + 1) || a.pos != b.pos || a.l0 != b.l0 || a.l1 != b.l1 || W.slot[i] != W.slot[i + 1]) return false;
+            if (((R.a1 >> i) & 1u) != ((R.a1 >> (i + 1)) & 1u) || ((R.a2 >> i) & 1u) != ((R.a2 >> (i + 1)) & 1u)) return false;
+            for (int x = 0; x < a.l0 + a.l1; ++x) if (c.alle[a.aoff + x] != c.alle[b.aoff + x]) return false;
+        }
+        return true;
     }
 
     AVK_HD static int popc16(u32 v) { v &= 0xffffu; int cnt = 0; while (v) { v &= v - 1; ++cnt; } return cnt; }
