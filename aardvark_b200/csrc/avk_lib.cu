@@ -1268,6 +1268,7 @@ struct avk_ctx {
     // variant table and bytes [p_base, ..) of its allele pool.  Per-variant device pointers are biased by these bases so
     // that kernels index them with the caller's own (global) indices: a contiguous bin needs no re-basing on the host.
     bool have_batch = false;
+    bool ids_resident = false;      // the resident batch was built on the device (avk_build_regions*): its region ids are in `region_id`
     bool have_result = false, result_has_rows = false;
     u64 lo = 0, n_regions = 0, v_base = 0, n_variants = 0, p_base = 0, pool_bytes = 0;
     u64 seq_base = 0, strat_base = 0;
@@ -1645,7 +1646,7 @@ static int upload_batch(avk_ctx *ctx, const avk_region_batch *b, BinScan &sc) {
     if (ref_of(ctx)->contig_bufs.empty()) { ctx->err = "avk_set_reference has not been called"; return AVK_ERR_NO_REFERENCE; }
     const u64 lo = sc.lo, n = sc.hi - sc.lo, K = b->n_inputs, v0 = sc.v0, nv = sc.v1 - sc.v0;
     const avk_variant_table &t = b->variants;
-    ctx->have_batch = false; ctx->have_result = false;
+    ctx->have_batch = false; ctx->have_result = false; ctx->ids_resident = false;
     UPLOAD(ctx->contig, b->contig + lo, 4 * n);
     UPLOAD(ctx->start, b->start + lo, 4 * n);
     UPLOAD(ctx->end, b->end + lo, 4 * n);
@@ -2691,10 +2692,10 @@ static int build_regions_impl(avk_ctx *ctx, const avk_callsets *in, const uint32
         }
     }
     if (sum_alle >= 0xffffffffull) { ctx->err = "avk_build_regions: allele bytes exceed 4 GiB"; return AVK_ERR_INVALID; }
-    ctx->have_batch = false; ctx->have_result = false;
+    ctx->have_batch = false; ctx->have_result = false; ctx->ids_resident = false;
     ctx->lo = 0; ctx->v_base = 0; ctx->p_base = 0; ctx->pool_bytes = 0;
     *n_regions_out = 0; *n_variants_out = 0;
-    if (nv == 0) { ctx->n_regions = 0; ctx->n_variants = 0; ctx->n_inputs = (u32)K; ctx->max_allele = 1; ctx->pool_len = 0; ctx->have_batch = true; ENSURE(ctx->var_off, 8); CK(cudaMemsetAsync(ctx->var_off.p, 0, 8, ctx->stream)); return AVK_OK; }
+    if (nv == 0) { ctx->n_regions = 0; ctx->n_variants = 0; ctx->n_inputs = (u32)K; ctx->max_allele = 1; ctx->pool_len = 0; ctx->have_batch = ctx->ids_resident = true; ENSURE(ctx->var_off, 8); CK(cudaMemsetAsync(ctx->var_off.p, 0, 8, ctx->stream)); return AVK_OK; }
     const unsigned g = (unsigned)((nv + 255) / 256);
     u64 *key = (u64 *)rb[T_KEY].p, *key_s = (u64 *)rb[T_KEY_S].p, *vend = (u64 *)rb[T_VEND].p, *pmax = (u64 *)rb[T_PMAX].p;
     u32 *idx = (u32 *)rb[T_IDX].p, *idx_s = (u32 *)rb[T_IDX_S].p, *flag = (u32 *)rb[T_FLAG].p, *cid = (u32 *)rb[T_CID].p, *perm = (u32 *)rb[T_PERM].p, *ivl = (u32 *)rb[T_IVL].p;
@@ -2756,7 +2757,7 @@ static int build_regions_impl(avk_ctx *ctx, const avk_callsets *in, const uint32
     }
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->n_regions = n; ctx->n_variants = nvalid; ctx->n_inputs = (u32)K; ctx->max_allele = mx; ctx->pool_len = kept_bytes; ctx->pool_bytes = kept_bytes;
-    ctx->have_batch = true;
+    ctx->have_batch = ctx->ids_resident = true;
     *n_regions_out = n; *n_variants_out = nvalid;
     return AVK_OK;
 }
@@ -3388,19 +3389,16 @@ __global__ void __launch_bounds__(128) k_bgzf_pack(const u8 *pay, const u32 *c_l
     const u8 *src = pay + (u64)k * BGZF_PAY_STRIDE;
     for (u32 i = threadIdx.x; i < c; i += blockDim.x) dst[18 + i] = src[i];
 }
-extern "C" int avk_bgzf_compress(avk_ctx *ctx, const uint8_t *text, uint64_t len, uint8_t *out, uint64_t cap, uint64_t *out_len) {
-    if (!ctx) return AVK_ERR_INVALID;
-    if ((!text && len) || !out_len) { ctx->err = "avk_bgzf_compress: bad arguments"; return AVK_ERR_INVALID; }
-    const u64 n_chunks = (len + avk_inflate::DEFLATE_CHUNK - 1) / avk_inflate::DEFLATE_CHUNK;
-    if (n_chunks >= 0x7fffffffull) { ctx->err = "avk_bgzf_compress: text too long for one call"; return AVK_ERR_INVALID; }
-    if (!out) { *out_len = len + 31 * n_chunks + 28; return AVK_OK; }        // upper bound: every chunk stored
-    CK(cudaSetDevice(ctx->device));
+static u64 bgzf_chunks(u64 len) { return (len + avk_inflate::DEFLATE_CHUNK - 1) / avk_inflate::DEFLATE_CHUNK; }
+static u64 bgzf_bound(u64 len) { return len + 31 * bgzf_chunks(len) + 28; }         // upper bound: every chunk stored, EOF marker
+enum { C_TEXT = V_TEXT, C_PAY = V_GZ, C_LEN = V_NOUT, C_CRC = V_NBYTES, C_OFF = V_STARTS, C_OUT = V_POOL };   // the compressor's rb slots
+// The `len` bytes of text already in rb[V_TEXT] -> BGZF members of 0xff00 input bytes (+ the EOF marker when eof) in `out`.
+static int bgzf_compress_device(avk_ctx *ctx, u64 len, bool eof, uint8_t *out, uint64_t cap, uint64_t *out_len) {
     DevBuf *rb = ctx->rb;
-    enum { C_TEXT = V_TEXT, C_PAY = V_GZ, C_LEN = V_NOUT, C_CRC = V_NBYTES, C_OFF = V_STARTS, C_OUT = V_POOL };
+    const u64 n_chunks = bgzf_chunks(len);
     std::vector<u64> m_off(n_chunks + 2, 0);
     std::vector<u32> c_len(n_chunks);
     if (n_chunks) {
-        UPLOAD(rb[C_TEXT], text, len);
         ENSURE(rb[C_PAY], n_chunks * (u64)BGZF_PAY_STRIDE);
         ENSURE(rb[C_LEN], 4 * n_chunks); ENSURE(rb[C_CRC], 4 * n_chunks);
         CK(cudaFuncSetAttribute(k_bgzf_deflate, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BGZF_DEF_SMEM));
@@ -3413,18 +3411,225 @@ extern "C" int avk_bgzf_compress(avk_ctx *ctx, const uint8_t *text, uint64_t len
     }
     for (u64 k = 0; k < n_chunks; ++k) m_off[k + 1] = m_off[k] + 18 + c_len[k] + 8;
     m_off[n_chunks + 1] = m_off[n_chunks] + 28;
-    const u64 total = m_off[n_chunks + 1];
+    const u64 total = m_off[n_chunks + (eof ? 1 : 0)];
     *out_len = total;
-    if (total > cap) { ctx->err = "avk_bgzf_compress: output capacity too small"; return AVK_ERR_OOM; }
+    if (total > cap) { ctx->err = "BGZF output capacity too small"; return AVK_ERR_OOM; }
+    if (total == 0) return AVK_OK;
     UPLOAD(rb[C_OFF], m_off.data(), 8 * m_off.size());
     ENSURE(rb[C_OUT], total);
-    k_bgzf_pack<<<(unsigned)(n_chunks + 1), 128, 0, ctx->stream>>>((const u8 *)rb[C_PAY].p, (const u32 *)rb[C_LEN].p, (const u32 *)rb[C_CRC].p, (const u64 *)rb[C_OFF].p, len,
-                                                                    (u32)n_chunks, (u8 *)rb[C_OUT].p);
+    k_bgzf_pack<<<(unsigned)(n_chunks + (eof ? 1 : 0)), 128, 0, ctx->stream>>>((const u8 *)rb[C_PAY].p, (const u32 *)rb[C_LEN].p, (const u32 *)rb[C_CRC].p,
+                                                                                (const u64 *)rb[C_OFF].p, len, (u32)n_chunks, (u8 *)rb[C_OUT].p);
     ctx->launches += 1;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(out, rb[C_OUT].p, total, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return AVK_OK;
+}
+extern "C" int avk_bgzf_compress(avk_ctx *ctx, const uint8_t *text, uint64_t len, uint8_t *out, uint64_t cap, uint64_t *out_len) {
+    if (!ctx) return AVK_ERR_INVALID;
+    if ((!text && len) || !out_len) { ctx->err = "avk_bgzf_compress: bad arguments"; return AVK_ERR_INVALID; }
+    if (bgzf_chunks(len) >= 0x7fffffffull) { ctx->err = "avk_bgzf_compress: text too long for one call"; return AVK_ERR_INVALID; }
+    if (!out) { *out_len = bgzf_bound(len); return AVK_OK; }
+    CK(cudaSetDevice(ctx->device));
+    if (len) UPLOAD(ctx->rb[C_TEXT], text, len);
+    return bgzf_compress_device(ctx, len, true, out, cap, out_len);
+}
+
+// ---- labelled VCF records of the resident compare, formatted on the device (avk_writers.h::vcf_records_text) ----------------
+// Count pass (one thread per region: records of the side, contig check) -> 64-bit scan -> length pass (one thread per record)
+// -> 64-bit scan -> write pass into rb[V_TEXT] after the header -> bgzf_compress_device.  Alleles longer than RW_LONG bytes
+// are copied by the whole warp, so an SV allele (or one of the 16 MiB scan_bin admits) does not hold up its warp's other lines.
+enum { W_CNT = V_VOFF, W_LEN = V_BOFF, W_NAMES = V_NAMES, W_MISC = V_MISC, W_REG = V_C, W_RID = V_POS };   // off the compressor's slots
+enum { RW_LONG = 32 };
+struct RecView {
+    const u64 *var_off, *rid;
+    const u32 *contig, *pos, *aoff, *l0, *l1;
+    const u8 *zyg, *pool, *cls, *exp, *obs;
+    const u64 *name_off;                 // [n_contigs + 1], the packed names follow
+    const char *names;
+    u32 K, side;
+};
+__device__ __forceinline__ u32 rw_digits(u64 x) { u32 d = 1; while (x >= 10) { x /= 10; ++d; } return d; }
+__device__ __forceinline__ u8 *rw_put_u64(u8 *o, u64 x, u32 d) { for (u32 k = d; k-- > 0; x /= 10) o[k] = (u8)('0' + x % 10); return o + d; }
+__device__ __forceinline__ u8 *rw_put_str(u8 *o, const char *s, u32 n) { for (u32 k = 0; k < n; ++k) o[k] = (u8)s[k]; return o + n; }
+// GT string (PhasedZygosity, variant_categorizer.rs:190-197) and BD label (Classification) of a record, as the host writer picks them
+__device__ __forceinline__ const char *rw_gt(u8 z, u32 &n) {
+    const char *s = z == 1 ? "0/0" : z == 2 ? "0/1" : z == 3 ? "0|1" : z == 4 ? "1|0" : z == 5 ? "1/1" : ".";
+    n = z >= 1 && z <= AVK_ZYG_HOM_ALT ? 3 : 1;
+    return s;
+}
+__device__ __forceinline__ const char *rw_bd(u8 c, u32 &n) {
+    n = c == 1 || c == 2 || c == 3 ? 2 : 3;
+    return c == 1 ? "TP" : c == 2 ? "FN" : c == AVK_CLASS_FP ? "FP" : "UNK";
+}
+// one allele copied by the whole warp, eight loads in flight per lane (the source and the text never overlap)
+__device__ __forceinline__ void rw_warp_copy(u8 *__restrict__ dst, const u8 *__restrict__ src, u32 n, int lane) {
+    for (u32 k = lane; k < n; k += 256) {
+        u8 b[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) b[j] = k + 32 * j < n ? src[k + 32 * j] : 0;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) if (k + 32 * j < n) dst[k + 32 * j] = b[j];
+    }
+}
+static __device__ const char RW_MID[] ="\t.\t.\t.\tGT:BD:EA:OA:RI\t";       // ALT | QUAL FILTER INFO FORMAT | sample
+enum { RW_MID_LEN = 22 };
+
+__global__ void __launch_bounds__(256) k_rw_count(RecView w, u64 n, u32 n_contigs, u64 *cnt, unsigned long long *bad) {
+    const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r > n) return;
+    if (r == n) { cnt[n] = 0; return; }
+    cnt[r] = w.var_off[r * w.K + w.side + 1] - w.var_off[r * w.K + w.side];
+    if (w.contig[r] >= n_contigs) atomicMax(bad, 1ull);
+}
+// record i of the side -> (region r, variant v); rec_off = exclusive scan of the per-region counts, [n + 1]
+__device__ __forceinline__ u64 rw_region(const u64 *rec_off, u64 n, u64 i) {
+    u64 lo = 0, hi = n;                                          // last r with rec_off[r] <= i (empty regions share offsets)
+    while (hi - lo > 1) { const u64 m = (lo + hi) >> 1; if (rec_off[m] <= i) lo = m; else hi = m; }
+    return lo;
+}
+__global__ void __launch_bounds__(256) k_rw_len(RecView w, u64 n, u64 n_rec, const u64 *rec_off, u32 *reg, u64 *len) {
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i > n_rec) return;
+    if (i == n_rec) { len[n_rec] = 0; return; }
+    const u64 r = rw_region(rec_off, n, i);
+    const u64 v = w.var_off[r * w.K + w.side] + (i - rec_off[r]);
+    const u32 c = w.contig[r];
+    const int32_t ri = (int32_t)(u32)w.rid[r];
+    u32 ng, nb;
+    rw_gt(w.zyg[v], ng); rw_bd(w.cls[v], nb);
+    reg[i] = (u32)r;
+    len[i] = (w.name_off[c + 1] - w.name_off[c]) + 1 + rw_digits((u64)w.pos[v] + 1) + 3 + w.l0[v] + 1 + w.l1[v] + RW_MID_LEN + ng + 1 + nb + 1 +
+             rw_digits(w.exp[v]) + 1 + rw_digits(w.obs[v]) + 1 + (ri < 0 ? 1 : 0) + rw_digits(ri < 0 ? (u64)(-(int64_t)ri) : (u64)ri) + 1;
+}
+// off = exclusive scan of the line lengths; line i starts at text + base + off[i]
+__global__ void __launch_bounds__(256) k_rw_write(RecView w, u64 n_rec, const u32 *reg, const u64 *rec_off, const u64 *off, u64 base, u8 *text) {
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool act = i < n_rec;
+    u64 a0_at = 0, a1_at = 0, src = 0;
+    u32 l0 = 0, l1 = 0;
+    if (act) {
+        const u64 r = reg[i];
+        const u64 v = w.var_off[r * w.K + w.side] + (i - rec_off[r]);
+        const u32 c = w.contig[r];
+        u8 *o = text + base + off[i];
+        o = rw_put_str(o, w.names + w.name_off[c], (u32)(w.name_off[c + 1] - w.name_off[c]));
+        *o++ = '\t';
+        const u64 p = (u64)w.pos[v] + 1;
+        o = rw_put_u64(o, p, rw_digits(p));
+        *o++ = '\t'; *o++ = '.'; *o++ = '\t';
+        l0 = w.l0[v]; l1 = w.l1[v];
+        src = (u64)(uintptr_t)(w.pool + w.aoff[v]);
+        a0_at = (u64)(o - text);
+        if (l0 <= RW_LONG) rw_put_str(o, (const char *)src, l0);
+        o += l0;
+        *o++ = '\t';
+        a1_at = (u64)(o - text);
+        if (l1 <= RW_LONG) rw_put_str(o, (const char *)src + l0, l1);
+        o += l1;
+        o = rw_put_str(o, RW_MID, RW_MID_LEN);
+        u32 ng, nb;
+        const char *gt = rw_gt(w.zyg[v], ng), *bd = rw_bd(w.cls[v], nb);
+        o = rw_put_str(o, gt, ng); *o++ = ':';
+        o = rw_put_str(o, bd, nb); *o++ = ':';
+        o = rw_put_u64(o, w.exp[v], rw_digits(w.exp[v])); *o++ = ':';
+        o = rw_put_u64(o, w.obs[v], rw_digits(w.obs[v])); *o++ = ':';
+        const int32_t ri = (int32_t)(u32)w.rid[r];                   // `region_id as i32` (:214)
+        if (ri < 0) *o++ = '-';
+        const u64 ra = ri < 0 ? (u64)(-(int64_t)ri) : (u64)ri;
+        o = rw_put_u64(o, ra, rw_digits(ra));
+        *o = '\n';
+    }
+    const int lane = lane_id();
+    for (u32 m = __ballot_sync(AVK_FULL, act && (l0 > RW_LONG || l1 > RW_LONG)); m; m &= m - 1) {
+        const int s = __ffs(m) - 1;
+        const u8 *sp = (const u8 *)(uintptr_t)__shfl_sync(AVK_FULL, src, s);
+        const u32 n0 = __shfl_sync(AVK_FULL, l0, s), n1 = __shfl_sync(AVK_FULL, l1, s);
+        const u64 d0 = __shfl_sync(AVK_FULL, a0_at, s), d1 = __shfl_sync(AVK_FULL, a1_at, s);
+        if (n0 > RW_LONG) rw_warp_copy(text + d0, sp, n0, lane);
+        if (n1 > RW_LONG) rw_warp_copy(text + d1, sp + n0, n1, lane);
+    }
+}
+
+extern "C" int avk_compare_records_bgzf(avk_ctx *ctx, uint32_t side, const char *const *contig_names, uint32_t n_contigs, const uint64_t *region_id,
+                                        const uint8_t *header, uint64_t header_len, int eof, uint8_t *out, uint64_t cap, uint64_t *out_len) {
+    if (!ctx) return AVK_ERR_INVALID;
+    if (!ctx->have_batch || !ctx->have_result) { ctx->err = "avk_compare_records_bgzf: no compare result is resident (run avk_compare_run_resident first)"; return AVK_ERR_INVALID; }
+    if (side >= ctx->n_inputs || (!contig_names && n_contigs) || (!header && header_len) || !out_len) { ctx->err = "avk_compare_records_bgzf: bad arguments"; return AVK_ERR_INVALID; }
+    if (!region_id && !ctx->ids_resident) { ctx->err = "avk_compare_records_bgzf: the batch was uploaded, so its region ids must be given"; return AVK_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->device));
+    DevBuf *rb = ctx->rb;
+    const u64 n = ctx->n_regions, K = ctx->n_inputs;
+    std::vector<u64> name_tab(n_contigs + 1, 0);
+    std::string packed;
+    for (u32 c = 0; c < n_contigs; ++c) {
+        if (!contig_names[c]) { ctx->err = "avk_compare_records_bgzf: null contig name"; return AVK_ERR_INVALID; }
+        packed += contig_names[c];
+        name_tab[c + 1] = packed.size();
+    }
+    const size_t tab_bytes = 8 * name_tab.size();
+    ENSURE(rb[W_NAMES], tab_bytes + packed.size());
+    CK(cudaMemcpyAsync(rb[W_NAMES].p, name_tab.data(), tab_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    if (!packed.empty()) CK(cudaMemcpyAsync((u8 *)rb[W_NAMES].p + tab_bytes, packed.data(), packed.size(), cudaMemcpyHostToDevice, ctx->stream));
+    const DevBatch db = dev_batch(ctx);
+    RecView w;
+    w.var_off = db.var_off; w.contig = db.contig; w.pos = db.pos; w.aoff = db.aoff; w.l0 = db.l0; w.l1 = db.l1; w.zyg = db.zyg; w.pool = db.pool;
+    w.cls = biased<const u8>(ctx->vcls, ctx->v_base); w.exp = biased<const u8>(ctx->vexp, ctx->v_base); w.obs = biased<const u8>(ctx->vobs, ctx->v_base);
+    w.name_off = (const u64 *)rb[W_NAMES].p; w.names = (const char *)rb[W_NAMES].p + tab_bytes;
+    w.K = (u32)K; w.side = side;
+    if (region_id) {                                              // the caller's ids of the resident bin [lo, lo + n)
+        UPLOAD(rb[W_RID], region_id + ctx->lo, 8 * n);
+        w.rid = (const u64 *)rb[W_RID].p;
+    } else {
+        w.rid = (const u64 *)ctx->region_id.p;
+    }
+    // count pass and the scan of the per-region record counts
+    ENSURE(rb[W_MISC], 64);
+    unsigned long long *d_misc = (unsigned long long *)rb[W_MISC].p;     // [0] contig out of range
+    ENSURE(rb[W_CNT], 8 * (n + 1));
+    u64 *rec_off = (u64 *)rb[W_CNT].p;
+    CK(cudaMemsetAsync(d_misc, 0, 8, ctx->stream));
+    size_t need = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, need, rec_off, rec_off, n + 1, ctx->stream);
+    ENSURE(ctx->scan_tmp, need);
+    k_rw_count<<<(unsigned)((n + 1 + 255) / 256), 256, 0, ctx->stream>>>(w, n, n_contigs, rec_off, d_misc);
+    CK(cub::DeviceScan::ExclusiveSum(ctx->scan_tmp.p, need, rec_off, rec_off, n + 1, ctx->stream));
+    unsigned long long h[2] = {0, 0};
+    CK(cudaMemcpyAsync(&h[0], d_misc, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&h[1], rec_off + n, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->launches += 2;
+    CK(cudaGetLastError());
+    if (h[0]) { ctx->err = "avk_compare_records_bgzf: a region's contig is not below n_contigs"; return AVK_ERR_INVALID; }
+    const u64 n_rec = h[1];
+    // length pass and the scan of the line lengths (64-bit counts and offsets throughout)
+    ENSURE(rb[W_LEN], 8 * (n_rec + 1));
+    ENSURE(rb[W_REG], 4 * n_rec);
+    u64 *off = (u64 *)rb[W_LEN].p;
+    u32 *reg = (u32 *)rb[W_REG].p;
+    need = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, need, off, off, n_rec + 1, ctx->stream);
+    ENSURE(ctx->scan_tmp, need);
+    k_rw_len<<<(unsigned)((n_rec + 1 + 255) / 256), 256, 0, ctx->stream>>>(w, n, n_rec, rec_off, reg, off);
+    CK(cub::DeviceScan::ExclusiveSum(ctx->scan_tmp.p, need, off, off, n_rec + 1, ctx->stream));
+    u64 body = 0;
+    CK(cudaMemcpyAsync(&body, off + n_rec, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->launches += 2;
+    CK(cudaGetLastError());
+    const u64 len = header_len + body;
+    if (bgzf_chunks(len) >= 0x7fffffffull) { ctx->err = "avk_compare_records_bgzf: text too long for one call"; return AVK_ERR_INVALID; }
+    if (!out) { *out_len = bgzf_bound(len); return AVK_OK; }
+    // header + lines into rb[V_TEXT], then the compressor
+    ENSURE(rb[C_TEXT], len);
+    u8 *text = (u8 *)rb[C_TEXT].p;
+    if (header_len) CK(cudaMemcpyAsync(text, header, header_len, cudaMemcpyHostToDevice, ctx->stream));
+    if (n_rec) {
+        k_rw_write<<<(unsigned)((n_rec + 255) / 256), 256, 0, ctx->stream>>>(w, n_rec, reg, rec_off, off, header_len, text);
+        ctx->launches += 1;
+        CK(cudaGetLastError());
+    }
+    return bgzf_compress_device(ctx, len, eof != 0, out, cap, out_len);
 }
 
 extern "C" int avk_vcf_parse_bgzf(avk_ctx *ctx, const uint8_t *gz, uint64_t gz_len, int verify_crc, const char *const *contig_names, uint32_t n_contigs,

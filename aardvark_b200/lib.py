@@ -110,6 +110,7 @@ EXPORTED_SYMBOLS = [
     "avk_compare_batch_range", "avk_compare_batch_multi", "avk_merge_batch_multi", "avk_partition_regions", "avk_compare_upload_range",
     "avk_compare_result_device", "avk_set_stratifications", "avk_create_lane",
     "avk_merge_records_write", "avk_merge_regions_write", "avk_merge_summary_write", "avk_bgzf_inflate", "avk_vcf_parse_bgzf", "avk_bgzf_compress", "avk_spec_profile",
+    "avk_compare_records_bgzf",
 ]
 
 

@@ -120,3 +120,26 @@ def bgzf_compress(solver, text: bytes) -> bytes:
     buf = C.create_string_buffer(int(n.value) + 1)
     solver._check(lib.avk_bgzf_compress(solver._ctx, text, len(text), buf, int(n.value), C.byref(n)), "avk_bgzf_compress")
     return buf.raw[:int(n.value)]
+
+
+def _records_bgzf_fn(lib):
+    lib.avk_compare_records_bgzf.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_char_p), C.c_uint32, C.POINTER(C.c_uint64), C.c_char_p,
+                                             C.c_uint64, C.c_int, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+    return lib.avk_compare_records_bgzf
+
+
+def vcf_records_bgzf(solver, side, contig_names, header: bytes = b"", region_ids=None, eof=True) -> bytes:
+    """avk_compare_records_bgzf: truth.vcf.gz (side 0) / query.vcf.gz (side 1) of the solver's resident compare result,
+    formatted and compressed on the device -- the same bytes as bgzf_compress(solver, header + vcf_record_lines(...)).
+    region_ids: the ids of the batch given to upload() (the whole batch's array; the resident bin's part is read), None
+    after build_regions().  eof=False leaves out the EOF marker so that the next bin's file can be appended."""
+    fn = _records_bgzf_fn(solver._lib)
+    names = (C.c_char_p * max(len(contig_names), 1))(*[n.encode() for n in contig_names])
+    rid = None if region_ids is None else np.ascontiguousarray(region_ids, dtype=np.uint64)
+    rid_p = abi.ptr(rid)
+    n = C.c_uint64(0)
+    call = lambda buf, cap: fn(solver._ctx, side, names, len(contig_names), rid_p, header, len(header), 1 if eof else 0, buf, cap, C.byref(n))
+    solver._check(call(None, 0), "avk_compare_records_bgzf")
+    out = np.empty(int(n.value), dtype=np.uint8)                 # an upper bound; pages past the compressed size are never touched
+    solver._check(call(out.ctypes.data, out.size), "avk_compare_records_bgzf")
+    return out[:int(n.value)].tobytes()

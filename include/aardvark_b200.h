@@ -412,6 +412,19 @@ int avk_summary_write(const uint64_t *totals, const uint8_t *metrics, uint32_t n
 int avk_vcf_records_write(const avk_region_batch *batch, uint32_t side, const char *const *contig_names, uint32_t n_contigs,
                           const uint8_t *var_class, const uint8_t *var_expected, const uint8_t *var_observed, uint64_t lo, uint64_t hi,
                           char *buf, uint64_t cap, uint64_t *len);
+/* The labelled records of input `side` (0 truth, 1 query) of the resident compare batch, formatted and BGZF-compressed
+ * on the device: out = a BGZF file whose inflated text is header[0..header_len) followed by exactly the lines
+ * avk_vcf_records_write(batch, side, contig_names, n_contigs, var_class, var_expected, var_observed, lo, lo + n) returns
+ * for the resident bin [lo, lo + n) and the last result (valid wherever avk_compare_download would succeed).  With eof != 0
+ * the file is byte for byte avk_bgzf_compress(header || those lines); eof == 0 leaves out the 28-byte EOF member, so that
+ * the files of consecutive bins (the header on the first only, eof on the last only) concatenate into one valid file.
+ * region_id: the caller's host array, indexed like the batch given to avk_compare_upload[_range] (elements lo .. lo+n-1
+ * are read); NULL when the resident batch was built by avk_build_regions[_bed], whose ids are on the device.
+ * A region whose contig is >= n_contigs fails the call (AVK_ERR_INVALID), as in avk_vcf_records_write.
+ * out == NULL: *out_len = an upper bound of the size.  Otherwise cap < size -> AVK_ERR_OOM with *out_len = the exact size. */
+int avk_compare_records_bgzf(avk_ctx *ctx, uint32_t side, const char *const *contig_names, uint32_t n_contigs,
+                             const uint64_t *region_id, const uint8_t *header, uint64_t header_len, int eof,
+                             uint8_t *out, uint64_t cap, uint64_t *out_len);
 
 /* The outputs of `aardvark merge` that are functions of avk_merge_out (host only; regions with status != 0 are skipped as
  * src/main.rs:507-524 skips failed regions; `result->status` may be NULL = all solved):
