@@ -632,6 +632,11 @@ __device__ __noinline__ void coop_dwfa_body() {
     const bool to_full = J.to_full != 0;
     int *gw = (int *)(uintptr_t)J.wf;
     int e = J.ed, status = DWFA_OK;
+    if (e > e_cap) {      // resumed past what cur / nxt hold (an earlier update of this alignment spilled): straight back to the warp path
+        if (tid == 0) { J.status = DWFA_COOP_SPILL; J.cells = 0; }
+        __syncthreads();
+        return;
+    }
     unsigned long long matched = 0, cells = 0;
     bool flag = false;
 #pragma unroll 1
