@@ -1270,6 +1270,7 @@ struct avk_ctx {
     bool have_batch = false;
     bool ids_resident = false;      // the resident batch was built on the device (avk_build_regions*): its region ids are in `region_id`
     bool have_result = false, result_has_rows = false;
+    bool result_has_contain = false;   // the last pass filled st_mask (a resident run never computes containment)
     u64 lo = 0, n_regions = 0, v_base = 0, n_variants = 0, p_base = 0, pool_bytes = 0;
     u64 seq_base = 0, strat_base = 0;
     u32 n_inputs = 0;
@@ -1556,8 +1557,7 @@ extern "C" int avk_set_stratifications(avk_ctx *ctx, const avk_strat_intervals *
     UPLOAD(ctx->st_pmax, pmax.data(), 4 * n_iv);
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->st_n = in->n_strata; ctx->st_contigs = in->n_contigs;
-    for (auto &sb : ctx->sib) if (sb) { const int rc = avk_set_stratifications(sb, in); if (rc != AVK_OK) return rc; }
-    return AVK_OK;
+    return AVK_OK;           // the streamed sibling and the lanes read these tables through ref_of()
 }
 
 // ---- host-side batch validation ---------------------------------------------------------------------------------------
@@ -2117,6 +2117,7 @@ static int compare_launch(avk_ctx *ctx, const avk_compare_cfg *cfg, bool want_se
     if (rc != AVK_OK) return rc;
     CK(cudaEventRecord(ctx->ev[4], ctx->stream));
     ctx->result_has_rows = rows;
+    ctx->result_has_contain = R.want_contain;
     return queue_counter_copies(ctx);
 }
 
@@ -2179,6 +2180,11 @@ struct BinTotals {
 static int download_compare_async(avk_ctx *ctx, avk_compare_out *out, bool want_seq, u64 seq_bytes) {
     const u64 n = ctx->n_regions, nv = ctx->n_variants, lo = ctx->lo, vb = ctx->v_base;
     const cudaStream_t ds = ctx->dn ? ctx->dn : ctx->stream;
+    // st_mask holds whatever an earlier pass left there, possibly for a smaller batch
+    if (out->containment && n && !ctx->result_has_contain) {
+        ctx->err = "containment masks were not computed by this run (avk_compare_run_resident never computes them)";
+        return AVK_ERR_INVALID;
+    }
     if (ctx->dn) CK(cudaStreamWaitEvent(ctx->dn, ctx->ev_done, 0));
     DL(out->status ? out->status + lo : nullptr, ctx->status, 4 * n);
     DL(out->ed1 ? out->ed1 + lo : nullptr, ctx->ed1, 4 * n);
@@ -2192,7 +2198,7 @@ static int download_compare_async(avk_ctx *ctx, avk_compare_out *out, bool want_
     DL(out->var_observed ? out->var_observed + vb : nullptr, ctx->vobs, nv);
     DL(out->var_class ? out->var_class + vb : nullptr, ctx->vcls, nv);
     CK(cudaMemcpyAsync(ctx->h_pin + 256, ctx->totals.p, 8 * RED_COLS + 64, cudaMemcpyDeviceToHost, ds));
-    if (out->containment && ctx->st_mask.p) DL(out->containment + lo, ctx->st_mask, 8 * n);
+    if (out->containment) DL(out->containment + lo, ctx->st_mask, 8 * n);
     if (want_seq) {
         DL(out->seq_len + lo * 5, ctx->seq_len, 4 * 5 * n);
         DL(out->seq_pool + ctx->seq_base, ctx->seq_pool, seq_bytes);
@@ -2360,6 +2366,7 @@ static int compare_streamed(avk_ctx *ctx, const avk_region_batch *batch, const a
     CK(cudaSetDevice(ctx->device));
     for (avk_ctx *l : lanes) {
         l->dense_n = ctx->dense_n; l->thread_pop_budget = ctx->thread_pop_budget; l->thread_batch_min = ctx->thread_batch_min; l->use_spec_search = ctx->use_spec_search; l->use_thread_stage = ctx->use_thread_stage; l->sort_shapes = ctx->sort_shapes; l->thread_min_regions = ctx->thread_min_regions;
+        l->coop_arena0 = ctx->coop_arena0; l->coop_arena1 = ctx->coop_arena1; l->coop_cap_ints = ctx->coop_cap_ints; l->wide_b0 = ctx->wide_b0;
         for (auto &st : l->copy_streams) if (!st) CK(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
         l->up = l->copy_streams[0]; l->dn = l->copy_streams[1];
     }
@@ -2817,6 +2824,7 @@ extern "C" int avk_compare_run_resident(avk_ctx *ctx, const avk_compare_cfg *cfg
 extern "C" int avk_compare_download(avk_ctx *ctx, avk_compare_out *out) {
     if (!ctx) return AVK_ERR_INVALID;
     if (!out || !ctx->have_batch || !ctx->have_result) { ctx->err = "no compare result is resident (run avk_compare_run_resident first)"; return AVK_ERR_INVALID; }
+    if (strata_wanted(out)) { ctx->err = "avk_compare_download returns no stratified sums: request them from avk_compare_batch*"; return AVK_ERR_INVALID; }
     CK(cudaSetDevice(ctx->device));
     int rc = download_compare_async(ctx, out, false, 0);
     if (rc != AVK_OK) return rc;

@@ -445,7 +445,10 @@ int avk_merge_summary_write(const avk_region_batch *batch, const avk_merge_out *
 int avk_compare_upload(avk_ctx *ctx, const avk_region_batch *batch);
 int avk_compare_upload_range(avk_ctx *ctx, const avk_region_batch *batch, uint64_t lo, uint64_t hi);
 int avk_compare_run_resident(avk_ctx *ctx, const avk_compare_cfg *cfg);
-/* copies the resident bin's results into out->...[lo..hi) / [v_base..) of the caller's arrays */
+/* copies the resident bin's results into out->...[lo..hi) / [v_base..) of the caller's arrays.  AVK_ERR_INVALID when out
+ * asks for what the last pass did not compute: region_metrics after a run without AVK_CMP_KEEP_REGION_ROWS, containment
+ * after avk_compare_run_resident (which never computes it), and stratified sums (strat_totals with n_strata > 0) always:
+ * request those from avk_compare_batch*. */
 int avk_compare_download(avk_ctx *ctx, avk_compare_out *out);
 /* DEVICE addresses of the resident bin's results (valid until the next call on the context): what a
  * one-process-per-GPU run hands to its single NCCL gather, so that results travel GPU -> root GPU over
