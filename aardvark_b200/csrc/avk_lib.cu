@@ -21,6 +21,7 @@
 #include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_run_length_encode.cuh>
 #include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
 #include <thrust/iterator/counting_iterator.h>
@@ -1270,6 +1271,7 @@ struct avk_ctx {
     bool have_batch = false;
     bool ids_resident = false;      // the resident batch was built on the device (avk_build_regions*): its region ids are in `region_id`
     bool have_result = false, result_has_rows = false;
+    bool have_merge = false;        // the last pass was a merge: its result (status, m_cls, m_nidx, m_idx) is resident; cleared with have_result
     bool result_has_contain = false;   // the last pass filled st_mask (a resident run never computes containment)
     u64 lo = 0, n_regions = 0, v_base = 0, n_variants = 0, p_base = 0, pool_bytes = 0;
     u64 seq_base = 0, strat_base = 0;
@@ -1527,7 +1529,7 @@ extern "C" int avk_set_reference(avk_ctx *ctx, uint32_t n_contigs, const uint8_t
     UPLOAD(ctx->d_contig_ptr, ptrs.data(), sizeof(u8 *) * n_contigs);
     UPLOAD(ctx->d_contig_len, lens, sizeof(u64) * n_contigs);
     CK(cudaStreamSynchronize(ctx->stream));
-    ctx->have_result = false;
+    ctx->have_result = ctx->have_merge = false;
     return AVK_OK;
 }
 
@@ -1646,7 +1648,7 @@ static int upload_batch(avk_ctx *ctx, const avk_region_batch *b, BinScan &sc) {
     if (ref_of(ctx)->contig_bufs.empty()) { ctx->err = "avk_set_reference has not been called"; return AVK_ERR_NO_REFERENCE; }
     const u64 lo = sc.lo, n = sc.hi - sc.lo, K = b->n_inputs, v0 = sc.v0, nv = sc.v1 - sc.v0;
     const avk_variant_table &t = b->variants;
-    ctx->have_batch = false; ctx->have_result = false; ctx->ids_resident = false;
+    ctx->have_batch = false; ctx->have_result = ctx->have_merge = false; ctx->ids_resident = false;
     UPLOAD(ctx->contig, b->contig + lo, 4 * n);
     UPLOAD(ctx->start, b->start + lo, 4 * n);
     UPLOAD(ctx->end, b->end + lo, 4 * n);
@@ -2095,7 +2097,7 @@ static int compare_launch(avk_ctx *ctx, const avk_compare_cfg *cfg, bool want_se
     R.strat_idx = (strata && !strat_dev) ? biased<const u32>(ctx->strat_idx, ctx->strat_base) : nullptr;
     R.strat_mask = (strata && strat_dev) ? (const u64 *)ctx->st_mask.p : nullptr;
     R.want_contain = strat_dev || want_contain;
-    ctx->have_result = false;
+    ctx->have_result = ctx->have_merge = false;
 
     CK(cudaEventRecord(ctx->ev[0], ctx->stream));
     int rc = run_alt_ed(ctx, R.db);
@@ -2531,7 +2533,7 @@ static int compare_lanes(avk_ctx *ctx, const avk_region_batch *batch, const avk_
     int rc = ensure_lanes(ctx, n);
     if (rc != AVK_OK) return rc;
     rc = compare_bins_concurrent(ctx->lanes.data(), (uint32_t)n, batch, cfg, out);
-    ctx->have_batch = ctx->have_result = false;             // the owner holds one bin only: nothing "resident" to re-run or download
+    ctx->have_batch = ctx->have_result = ctx->have_merge = false;   // the owner holds one bin only: nothing "resident" to re-run or download
     // the owner's timings describe the call: the longest device pass of the lanes
     for (int i = 1; i < n; ++i) if (ctx->lanes[i]->last_ms[4] > ctx->last_ms[4]) for (int k = 0; k < 5; ++k) ctx->last_ms[k] = ctx->lanes[i]->last_ms[k];
     return rc;
@@ -2699,7 +2701,7 @@ static int build_regions_impl(avk_ctx *ctx, const avk_callsets *in, const uint32
         }
     }
     if (sum_alle >= 0xffffffffull) { ctx->err = "avk_build_regions: allele bytes exceed 4 GiB"; return AVK_ERR_INVALID; }
-    ctx->have_batch = false; ctx->have_result = false; ctx->ids_resident = false;
+    ctx->have_batch = false; ctx->have_result = ctx->have_merge = false; ctx->ids_resident = false;
     ctx->lo = 0; ctx->v_base = 0; ctx->p_base = 0; ctx->pool_bytes = 0;
     *n_regions_out = 0; *n_variants_out = 0;
     if (nv == 0) { ctx->n_regions = 0; ctx->n_variants = 0; ctx->n_inputs = (u32)K; ctx->max_allele = 1; ctx->pool_len = 0; ctx->have_batch = ctx->ids_resident = true; ENSURE(ctx->var_off, 8); CK(cudaMemsetAsync(ctx->var_off.p, 0, 8, ctx->stream)); return AVK_OK; }
@@ -2892,16 +2894,12 @@ extern "C" int avk_last_work(avk_ctx *ctx, avk_work_counters *out) {
     return AVK_OK;
 }
 
-// solve_merge_region over one contiguous bin [lo, hi) of the batch; results land in the caller's arrays at the bin's offsets
-static int merge_bin(avk_ctx *ctx, const avk_region_batch *batch, u64 lo, u64 hi, const avk_merge_cfg *cfg, avk_merge_out *out) {
-    CK(cudaSetDevice(ctx->device));
-    BinScan sc;
-    int rc = bin_range(ctx, batch, lo, hi, sc);
-    if (rc != AVK_OK) return rc;
-    rc = upload_batch(ctx, batch, sc);
-    if (rc != AVK_OK) return rc;
+// solve_merge_region over the resident batch: front stage, pair tasks and classification are queued on ctx->stream; the
+// result stays in status / m_cls / m_nidx / m_idx (merge_finish marks it resident)
+static int merge_launch(avk_ctx *ctx, const avk_merge_cfg *cfg) {
     const u64 n = ctx->n_regions;
     const u32 K = ctx->n_inputs;
+    ctx->have_result = ctx->have_merge = false;                 // the pass overwrites `status`, which a compare result owns too
     ENSURE(ctx->status, 4 * n); ENSURE(ctx->m_cls, n); ENSURE(ctx->m_nidx, n); ENSURE(ctx->m_idx, n * K);
     ENSURE(ctx->counters, 64); ENSURE(ctx->work_ctr, 64);
     CK(cudaMemsetAsync(ctx->work_ctr.p, 0, 64, ctx->stream));
@@ -2910,7 +2908,7 @@ static int merge_bin(avk_ctx *ctx, const avk_region_batch *batch, u64 lo, u64 hi
     mo.status = (int *)ctx->status.p; mo.cls = (u8 *)ctx->m_cls.p; mo.n_idx = (u8 *)ctx->m_nidx.p; mo.idx = (u8 *)ctx->m_idx.p;
     avk_merge_cfg c = *cfg;
     CK(cudaEventRecord(ctx->ev[0], ctx->stream));
-    rc = run_alt_ed(ctx, db);
+    int rc = run_alt_ed(ctx, db);
     if (rc != AVK_OK) return rc;
     CK(cudaEventRecord(ctx->ev[1], ctx->stream));
     const int sm = ctx->sm_count;
@@ -2942,19 +2940,82 @@ static int merge_bin(avk_ctx *ctx, const avk_region_batch *batch, u64 lo, u64 hi
         ctx->launches += 1;
         CK(cudaGetLastError());
     }
-    if (rc != AVK_OK) return rc;
     CK(cudaEventRecord(ctx->ev[2], ctx->stream));
     CK(cudaEventRecord(ctx->ev[3], ctx->stream));
     CK(cudaEventRecord(ctx->ev[4], ctx->stream));
+    return AVK_OK;
+}
+// the resident bin's merge result -> the caller's arrays at the bin's offsets (queued on ctx->stream)
+static int merge_queue_download(avk_ctx *ctx, avk_merge_out *out) {
+    const u64 n = ctx->n_regions, lo = ctx->lo, K = ctx->n_inputs;
     const cudaStream_t ds = ctx->stream;
     DL(out->status + lo, ctx->status, 4 * n);
     DL(out->classification ? out->classification + lo : nullptr, ctx->m_cls, n);
     DL(out->n_indices ? out->n_indices + lo : nullptr, ctx->m_nidx, n);
     DL(out->indices ? out->indices + lo * K : nullptr, ctx->m_idx, n * K);
+    return AVK_OK;
+}
+// waits for the pass (and any queued download) and reads its timings and work counters; the result is then resident
+static int merge_finish(avk_ctx *ctx) {
     CK(cudaMemcpyAsync(ctx->h_pin + 128, ctx->work_ctr.p, 40, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaEventRecord(ctx->ev_done, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    return fetch_timings(ctx);
+    const int rc = fetch_timings(ctx);
+    if (rc != AVK_OK) return rc;
+    ctx->have_merge = true;
+    return AVK_OK;
+}
+
+// solve_merge_region over one contiguous bin [lo, hi) of the batch; results land in the caller's arrays at the bin's offsets
+// and stay resident on the context
+static int merge_bin(avk_ctx *ctx, const avk_region_batch *batch, u64 lo, u64 hi, const avk_merge_cfg *cfg, avk_merge_out *out) {
+    CK(cudaSetDevice(ctx->device));
+    BinScan sc;
+    int rc = bin_range(ctx, batch, lo, hi, sc);
+    if (rc != AVK_OK) return rc;
+    rc = upload_batch(ctx, batch, sc);
+    if (rc != AVK_OK) return rc;
+    rc = merge_launch(ctx, cfg);
+    if (rc != AVK_OK) return rc;
+    rc = merge_queue_download(ctx, out);
+    if (rc != AVK_OK) return rc;
+    return merge_finish(ctx);
+}
+
+extern "C" int avk_merge_upload_range(avk_ctx *ctx, const avk_region_batch *batch, uint64_t lo, uint64_t hi) {
+    if (!ctx) return AVK_ERR_INVALID;
+    CK(cudaSetDevice(ctx->device));
+    int rc = validate_batch(ctx, batch, false);
+    if (rc != AVK_OK) return rc;
+    if (lo > hi || hi > batch->n_regions) { ctx->err = "region range outside the batch"; return AVK_ERR_INVALID; }
+    BinScan sc;
+    rc = bin_range(ctx, batch, lo, hi, sc);
+    if (rc != AVK_OK) return rc;
+    rc = upload_batch(ctx, batch, sc);
+    if (rc != AVK_OK) return rc;
+    CK(cudaStreamSynchronize(ctx->stream));
+    return AVK_OK;
+}
+
+extern "C" int avk_merge_run_resident(avk_ctx *ctx, const avk_merge_cfg *cfg) {
+    if (!ctx) return AVK_ERR_INVALID;
+    if (!cfg || !ctx->have_batch) { ctx->err = "avk_merge_run_resident: no resident batch (avk_merge_upload_range or avk_build_regions[_bed] first)"; return AVK_ERR_INVALID; }
+    if (ctx->n_inputs < 1 || ctx->n_inputs > 32) { ctx->err = "avk_merge_run_resident: unsupported n_inputs (1 .. 32)"; return AVK_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->device));
+    const int rc = merge_launch(ctx, cfg);
+    if (rc != AVK_OK) return rc;
+    return merge_finish(ctx);
+}
+
+extern "C" int avk_merge_download(avk_ctx *ctx, avk_merge_out *out) {
+    if (!ctx) return AVK_ERR_INVALID;
+    if (!ctx->have_batch || !ctx->have_merge) { ctx->err = "avk_merge_download: no merge result is resident (run avk_merge_run_resident first)"; return AVK_ERR_INVALID; }
+    if (!out || !out->status) { ctx->err = "avk_merge_download: null out/status"; return AVK_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->device));
+    const int rc = merge_queue_download(ctx, out);
+    if (rc != AVK_OK) return rc;
+    CK(cudaStreamSynchronize(ctx->stream));
+    return AVK_OK;
 }
 
 extern "C" int avk_merge_batch(avk_ctx *ctx, const avk_region_batch *batch, const avk_merge_cfg *cfg, avk_merge_out *out) {
@@ -3035,7 +3096,7 @@ extern "C" int avk_wfa_ed_batch(avk_ctx *ctx, uint64_t n_pairs, const uint8_t *p
     CK(cudaEventRecord(ctx->ev[2], ctx->stream));
     CK(cudaEventRecord(ctx->ev[3], ctx->stream));
     CK(cudaEventRecord(ctx->ev[4], ctx->stream));
-    ctx->have_result = false;
+    ctx->have_result = ctx->have_merge = false;
     CK(cudaMemcpyAsync(ed_out, ctx->pair_ed.p, 4 * n_pairs, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(ctx->h_pin + 128, ctx->work_ctr.p, 40, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaEventRecord(ctx->ev_done, ctx->stream));
@@ -3108,6 +3169,15 @@ extern "C" int avk_merge_summary_write(const avk_region_batch *batch, const avk_
     avk_writers::MergeView m;
     if (!input_labels || merge_view(batch, result, 0, false, m) != AVK_OK) return AVK_ERR_INVALID;
     return copy_text(avk_writers::merge_summary_text(batch, input_labels, m, csv ? ',' : '\t', header != 0), buf, cap, len);
+}
+extern "C" int avk_merge_summary_rows_write(const avk_merge_summary_row *rows, uint64_t n_rows, uint32_t n_inputs, const char *const *input_labels,
+                                            int csv, int header, char *buf, uint64_t cap, uint64_t *len) {
+    if ((!rows && n_rows) || !input_labels || n_inputs == 0 || n_inputs > 32) return AVK_ERR_INVALID;
+    for (uint64_t i = 0; i < n_rows; ++i)
+        if (rows[i].input >= n_inputs || !input_labels[rows[i].input] || (n_inputs < 32 && (rows[i].indices >> n_inputs))) return AVK_ERR_INVALID;
+    avk_writers::MergeSummaryCounts counts;
+    avk_writers::merge_summary_count_rows(counts, rows, n_rows);
+    return copy_text(avk_writers::merge_summary_format(counts, input_labels, csv ? ',' : '\t', header != 0), buf, cap, len);
 }
 
 // ---- VCF body text -> call-set table (SURVEY 8f N2, avk_vcf.cuh) -----------------------------------------------------------
@@ -3638,6 +3708,423 @@ extern "C" int avk_compare_records_bgzf(avk_ctx *ctx, uint32_t side, const char 
         CK(cudaGetLastError());
     }
     return bgzf_compress_device(ctx, len, eof != 0, out, cap, out_len);
+}
+
+// ---- outputs of the resident merge, formatted on the device (avk_writers.h::merge_records_text / merge_regions_text and the
+// keys of merge_summary_count_batch) --------------------------------------------------------------------------------------
+// passing.vcf.gz: count pass (one thread per region: records of the source input, length of the region's INFO text, checks)
+// -> scans of the record counts and of the INFO lengths -> the INFO text of every passing region into rb[M_INFO], built once
+// -> length pass (one thread per record) -> scan -> write pass, which copies the region's INFO into each of its lines ->
+// bgzf_compress_device.  INFO strings and alleles longer than RW_LONG bytes are copied by the whole warp, as in k_rw_write.
+// regions.bed / failed_regions.bed: one line per region, a length pass, a scan and a write pass.
+enum { M_IOFF = V_VT, M_INFO = V_ZY, M_KEY = V_RAW, M_KEY_S = V_AOFF, M_UNIQ = V_L0, M_RUNS = V_L1 };    // beside the compare writer's slots
+enum { MW_BAD_CONTIG = 1, MW_BAD_INDEX = 2 };
+struct MergeRecView {
+    const u64 *var_off, *rid;
+    const u32 *contig, *start, *end, *pos, *aoff, *l0, *l1;
+    const u8 *zyg, *vtype, *pool;
+    const int *status;
+    const u8 *cls, *n_idx, *idx;
+    const u64 *name_off, *label_off;     // [n_contigs + 1] and [K + 1] offsets into the packed names / labels
+    const char *names, *labels;
+    u32 K;
+};
+// avk_writers.h::merge_simple and merge_source
+__device__ __forceinline__ const char *mw_simple(u8 c, u32 &n) {
+    switch (c) {
+        case AVK_MERGE_NO_CONFLICT: n = 11; return "no_conflict";
+        case AVK_MERGE_MAJORITY_AGREE: n = 8; return "majority";
+        case AVK_MERGE_CONFLICT_SELECTION: n = 15; return "conflict_select";
+        case AVK_MERGE_BASEPAIR_IDENTICAL: n = 9; return "identical";
+        default: n = 9; return "different";
+    }
+}
+__device__ __forceinline__ int mw_source(const MergeRecView &w, u64 r) {
+    const u8 c = w.cls[r];
+    if (c == AVK_MERGE_BASEPAIR_IDENTICAL) return 0;
+    if (c == AVK_MERGE_DIFFERENT || w.n_idx[r] == 0) return -1;
+    return w.idx[r * w.K];
+}
+// the checks of avk_lib.cu::merge_view on one region: its contig has a name, its index list lies inside the inputs
+__device__ __forceinline__ u32 mw_check(const MergeRecView &w, u64 r, u32 n_contigs) {
+    u32 bad = w.contig[r] >= n_contigs ? (u32)MW_BAD_CONTIG : 0u;
+    const u32 ni = w.n_idx[r];
+    if (ni > w.K) bad |= MW_BAD_INDEX;
+    else for (u32 k = 0; k < ni; ++k) if (w.idx[r * w.K + k] >= w.K) bad |= MW_BAD_INDEX;
+    return bad;
+}
+__device__ __forceinline__ u32 mw_label_len(const MergeRecView &w, u32 k) { return (u32)(w.label_off[k + 1] - w.label_off[k]); }
+
+__global__ void __launch_bounds__(256) k_mw_count(MergeRecView w, u64 n, u32 n_contigs, u64 *cnt, u64 *ilen, unsigned long long *bad) {
+    const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r > n) return;
+    if (r == n) { cnt[n] = 0; ilen[n] = 0; return; }
+    const u32 b = mw_check(w, r, n_contigs);
+    if (b) atomicOr(bad, (unsigned long long)b);
+    u64 c = 0, il = 0;
+    const int src = b || w.status[r] != 0 ? -1 : mw_source(w, r);
+    if (src >= 0) c = w.var_off[r * w.K + src + 1] - w.var_off[r * w.K + src];
+    if (c) {                                                      // SOURCES=<labels>;MR=<reason>
+        u32 ns;
+        mw_simple(w.cls[r], ns);
+        il = 8 + 4 + ns;
+        if (w.cls[r] == AVK_MERGE_BASEPAIR_IDENTICAL) for (u32 k = 0; k < w.K; ++k) il += (k ? 1 : 0) + mw_label_len(w, k);
+        else for (u32 k = 0; k < w.n_idx[r]; ++k) il += (k ? 1 : 0) + mw_label_len(w, w.idx[r * w.K + k]);
+    }
+    cnt[r] = c;
+    ilen[r] = il;
+}
+// the INFO text of each region with records, at info + ioff[r] (ioff = exclusive scan of the INFO lengths)
+__global__ void __launch_bounds__(256) k_mw_info(MergeRecView w, u64 n, const u64 *ioff, u8 *info) {
+    const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n || ioff[r + 1] == ioff[r]) return;
+    u8 *o = info + ioff[r];
+    o = rw_put_str(o, "SOURCES=", 8);
+    const bool all = w.cls[r] == AVK_MERGE_BASEPAIR_IDENTICAL;
+    const u32 m = all ? w.K : w.n_idx[r];
+    for (u32 k = 0; k < m; ++k) {
+        if (k) *o++ = ',';
+        const u32 in = all ? k : w.idx[r * w.K + k];
+        o = rw_put_str(o, w.labels + w.label_off[in], mw_label_len(w, in));
+    }
+    o = rw_put_str(o, ";MR=", 4);
+    u32 ns;
+    const char *s = mw_simple(w.cls[r], ns);
+    rw_put_str(o, s, ns);
+}
+__global__ void __launch_bounds__(256) k_mw_len(MergeRecView w, u64 n, u64 n_rec, const u64 *rec_off, const u64 *ioff, u32 *reg, u64 *len) {
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i > n_rec) return;
+    if (i == n_rec) { len[n_rec] = 0; return; }
+    const u64 r = rw_region(rec_off, n, i);
+    const u64 v = w.var_off[r * w.K + mw_source(w, r)] + (i - rec_off[r]);
+    const u32 c = w.contig[r];
+    const int32_t ri = (int32_t)(u32)w.rid[r];
+    u32 ng;
+    rw_gt(w.zyg[v], ng);
+    reg[i] = (u32)r;
+    len[i] = (w.name_off[c + 1] - w.name_off[c]) + 1 + rw_digits((u64)w.pos[v] + 1) + 3 + w.l0[v] + 1 + w.l1[v] + 5 + (ioff[r + 1] - ioff[r]) + 7 +
+             ng + 1 + (ri < 0 ? 1 : 0) + rw_digits(ri < 0 ? (u64)(-(int64_t)ri) : (u64)ri) + 1;
+}
+// off = exclusive scan of the line lengths; line i starts at text + base + off[i]
+__global__ void __launch_bounds__(256) k_mw_write(MergeRecView w, u64 n_rec, const u32 *reg, const u64 *rec_off, const u64 *ioff, const u8 *info,
+                                                  const u64 *off, u64 base, u8 *text) {
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool act = i < n_rec;
+    u64 a0_at = 0, a1_at = 0, in_at = 0, src = 0, isrc = 0;
+    u32 l0 = 0, l1 = 0, li = 0;
+    if (act) {
+        const u64 r = reg[i];
+        const u64 v = w.var_off[r * w.K + mw_source(w, r)] + (i - rec_off[r]);
+        const u32 c = w.contig[r];
+        u8 *o = text + base + off[i];
+        o = rw_put_str(o, w.names + w.name_off[c], (u32)(w.name_off[c + 1] - w.name_off[c]));
+        *o++ = '\t';
+        const u64 p = (u64)w.pos[v] + 1;
+        o = rw_put_u64(o, p, rw_digits(p));
+        *o++ = '\t'; *o++ = '.'; *o++ = '\t';
+        l0 = w.l0[v]; l1 = w.l1[v];
+        src = (u64)(uintptr_t)(w.pool + w.aoff[v]);
+        a0_at = (u64)(o - text);
+        if (l0 <= RW_LONG) rw_put_str(o, (const char *)src, l0);
+        o += l0;
+        *o++ = '\t';
+        a1_at = (u64)(o - text);
+        if (l1 <= RW_LONG) rw_put_str(o, (const char *)src + l0, l1);
+        o += l1;
+        o = rw_put_str(o, "\t.\t.\t", 5);
+        li = (u32)(ioff[r + 1] - ioff[r]);
+        isrc = (u64)(uintptr_t)(info + ioff[r]);
+        in_at = (u64)(o - text);
+        if (li <= RW_LONG) rw_put_str(o, (const char *)isrc, li);
+        o += li;
+        o = rw_put_str(o, "\tGT:RI\t", 7);
+        u32 ng;
+        const char *gt = rw_gt(w.zyg[v], ng);
+        o = rw_put_str(o, gt, ng); *o++ = ':';
+        const int32_t ri = (int32_t)(u32)w.rid[r];                   // `region_id as i32`
+        if (ri < 0) *o++ = '-';
+        const u64 ra = ri < 0 ? (u64)(-(int64_t)ri) : (u64)ri;
+        o = rw_put_u64(o, ra, rw_digits(ra));
+        *o = '\n';
+    }
+    const int lane = lane_id();
+    for (u32 m = __ballot_sync(AVK_FULL, act && (l0 > RW_LONG || l1 > RW_LONG || li > RW_LONG)); m; m &= m - 1) {
+        const int s = __ffs(m) - 1;
+        const u8 *sp = (const u8 *)(uintptr_t)__shfl_sync(AVK_FULL, src, s), *ip = (const u8 *)(uintptr_t)__shfl_sync(AVK_FULL, isrc, s);
+        const u32 n0 = __shfl_sync(AVK_FULL, l0, s), n1 = __shfl_sync(AVK_FULL, l1, s), ni = __shfl_sync(AVK_FULL, li, s);
+        const u64 d0 = __shfl_sync(AVK_FULL, a0_at, s), d1 = __shfl_sync(AVK_FULL, a1_at, s), di = __shfl_sync(AVK_FULL, in_at, s);
+        if (n0 > RW_LONG) rw_warp_copy(text + d0, sp, n0, lane);
+        if (n1 > RW_LONG) rw_warp_copy(text + d1, sp + n0, n1, lane);
+        if (ni > RW_LONG) rw_warp_copy(text + di, ip, ni, lane);
+    }
+}
+// BED4 line of a solved region whose pass / fail state is `passing`: chrom, start, end, {reason}_{region id as u64}
+__global__ void __launch_bounds__(256) k_mr_len(MergeRecView w, u64 n, u32 n_contigs, int passing, u64 *len, unsigned long long *bad) {
+    const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r > n) return;
+    if (r == n) { len[n] = 0; return; }
+    const u32 b = mw_check(w, r, n_contigs);
+    if (b) atomicOr(bad, (unsigned long long)b);
+    u64 l = 0;
+    if (!b && w.status[r] == 0 && (mw_source(w, r) >= 0) == (passing != 0)) {
+        const u32 c = w.contig[r];
+        u32 ns;
+        mw_simple(w.cls[r], ns);
+        l = (w.name_off[c + 1] - w.name_off[c]) + 1 + rw_digits(w.start[r]) + 1 + rw_digits(w.end[r]) + 1 + ns + 1 + rw_digits(w.rid[r]) + 1;
+    }
+    len[r] = l;
+}
+__global__ void __launch_bounds__(256) k_mr_write(MergeRecView w, u64 n, const u64 *off, u8 *text) {
+    const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n || off[r + 1] == off[r]) return;
+    const u32 c = w.contig[r];
+    u8 *o = text + off[r];
+    o = rw_put_str(o, w.names + w.name_off[c], (u32)(w.name_off[c + 1] - w.name_off[c]));
+    *o++ = '\t';
+    o = rw_put_u64(o, w.start[r], rw_digits(w.start[r])); *o++ = '\t';
+    o = rw_put_u64(o, w.end[r], rw_digits(w.end[r])); *o++ = '\t';
+    u32 ns;
+    const char *s = mw_simple(w.cls[r], ns);
+    o = rw_put_str(o, s, ns); *o++ = '_';
+    o = rw_put_u64(o, w.rid[r], rw_digits(w.rid[r]));
+    *o = '\n';
+}
+// the summary key of every variant of the bin (avk_writers.h::merge_summary_count_batch): class << 56 | variant type << 48 |
+// input << 40 | index-list mask; ~0 for a variant of an unsolved region (it sorts last and is dropped)
+__global__ void __launch_bounds__(256) k_ms_keys(MergeRecView w, u64 n, u64 v_base, u64 nv, u64 *key, unsigned long long *bad) {
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nv) return;
+    const u64 v = v_base + i, nl = n * w.K;
+    u64 lo = 0, hi = nl;                                          // list j = r * K + k holds v: the last j with var_off[j] <= v
+    while (hi - lo > 1) { const u64 m = (lo + hi) >> 1; if (w.var_off[m] <= v) lo = m; else hi = m; }
+    const u64 r = lo / w.K, k = lo % w.K;
+    if (w.status[r] != 0) { key[i] = ~0ull; return; }
+    if (mw_check(w, r, 0xffffffffu)) atomicOr(bad, (unsigned long long)MW_BAD_INDEX);
+    const u8 c = w.cls[r];
+    const u8 *ix = w.idx + r * w.K;
+    u32 mask = 0;
+    if (c == AVK_MERGE_NO_CONFLICT || c == AVK_MERGE_MAJORITY_AGREE) { for (u32 j = 0; j < w.n_idx[r] && j < w.K; ++j) mask |= 1u << (ix[j] & 31); }
+    else if (c == AVK_MERGE_CONFLICT_SELECTION) mask = 1u << (ix[0] & 31);
+    key[i] = (u64)c << 56 | (u64)w.vtype[v] << 48 | k << 40 | mask;
+}
+
+// the resident merge result and batch as the writers read them; names and labels (when given) uploaded into rb[W_NAMES]
+static int merge_view_device(avk_ctx *ctx, const char *who, const char *const *contig_names, uint32_t n_contigs, const char *const *labels,
+                             const uint64_t *region_id, bool need_ids, MergeRecView &w) {
+    std::string &err = ctx->err;
+    if (!ctx->have_batch || !ctx->have_merge) { err = std::string(who) + ": no merge result is resident (run avk_merge_run_resident first)"; return AVK_ERR_INVALID; }
+    if (!contig_names && n_contigs) { err = std::string(who) + ": bad arguments"; return AVK_ERR_INVALID; }
+    if (need_ids && !region_id && !ctx->ids_resident) { err = std::string(who) + ": the batch was uploaded, so its region ids must be given"; return AVK_ERR_INVALID; }
+    const u64 n = ctx->n_regions, K = ctx->n_inputs;
+    std::vector<u64> tab(n_contigs + 1 + (labels ? K + 1 : 0), 0);
+    std::string packed;
+    for (u32 c = 0; c < n_contigs; ++c) {
+        if (!contig_names[c]) { err = std::string(who) + ": null contig name"; return AVK_ERR_INVALID; }
+        packed += contig_names[c];
+        tab[c + 1] = packed.size();
+    }
+    const u64 names_len = packed.size();
+    if (labels) {
+        u64 *lt = tab.data() + n_contigs + 1;
+        for (u64 k = 0; k < K; ++k) {
+            if (!labels[k]) { err = std::string(who) + ": null input label"; return AVK_ERR_INVALID; }
+            packed += labels[k];
+            lt[k + 1] = packed.size() - names_len;
+        }
+    }
+    DevBuf *rb = ctx->rb;
+    const size_t tab_bytes = 8 * tab.size();
+    ENSURE(rb[W_NAMES], tab_bytes + packed.size());
+    CK(cudaMemcpyAsync(rb[W_NAMES].p, tab.data(), tab_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    if (!packed.empty()) CK(cudaMemcpyAsync((u8 *)rb[W_NAMES].p + tab_bytes, packed.data(), packed.size(), cudaMemcpyHostToDevice, ctx->stream));
+    const DevBatch db = dev_batch(ctx);
+    w.var_off = db.var_off; w.contig = db.contig; w.start = db.start; w.end = db.end; w.pos = db.pos; w.aoff = db.aoff; w.l0 = db.l0; w.l1 = db.l1;
+    w.zyg = db.zyg; w.vtype = db.vtype; w.pool = db.pool;
+    w.status = (const int *)ctx->status.p; w.cls = (const u8 *)ctx->m_cls.p; w.n_idx = (const u8 *)ctx->m_nidx.p; w.idx = (const u8 *)ctx->m_idx.p;
+    w.name_off = (const u64 *)rb[W_NAMES].p; w.label_off = w.name_off + n_contigs + 1;
+    w.names = (const char *)rb[W_NAMES].p + tab_bytes; w.labels = w.names + names_len;
+    w.K = (u32)K;
+    w.rid = nullptr;
+    if (need_ids) {
+        if (region_id) {                                          // the caller's ids of the resident bin [lo, lo + n)
+            UPLOAD(rb[W_RID], region_id + ctx->lo, 8 * n);
+            w.rid = (const u64 *)rb[W_RID].p;
+        } else {
+            w.rid = (const u64 *)ctx->region_id.p;
+        }
+    }
+    return AVK_OK;
+}
+static int merge_bad(avk_ctx *ctx, const char *who, unsigned long long bad) {
+    if (bad & MW_BAD_CONTIG) { ctx->err = std::string(who) + ": a region's contig is not below n_contigs"; return AVK_ERR_INVALID; }
+    if (bad & MW_BAD_INDEX) { ctx->err = std::string(who) + ": a merge result's index list lies outside the inputs"; return AVK_ERR_INVALID; }
+    return AVK_OK;
+}
+
+extern "C" int avk_merge_records_bgzf(avk_ctx *ctx, const char *const *contig_names, uint32_t n_contigs, const char *const *input_labels,
+                                      const uint64_t *region_id, const uint8_t *header, uint64_t header_len, int eof,
+                                      uint8_t *out, uint64_t cap, uint64_t *out_len) {
+    static const char *who = "avk_merge_records_bgzf";
+    if (!ctx) return AVK_ERR_INVALID;
+    if (!input_labels || (!header && header_len) || !out_len) { ctx->err = std::string(who) + ": bad arguments"; return AVK_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->device));
+    MergeRecView w;
+    int rc = merge_view_device(ctx, who, contig_names, n_contigs, input_labels, region_id, true, w);
+    if (rc != AVK_OK) return rc;
+    DevBuf *rb = ctx->rb;
+    const u64 n = ctx->n_regions;
+    // count pass and the scans of the per-region record counts and INFO lengths
+    ENSURE(rb[W_MISC], 64);
+    unsigned long long *d_misc = (unsigned long long *)rb[W_MISC].p;     // [0] MW_BAD_* flags
+    ENSURE(rb[W_CNT], 8 * (n + 1)); ENSURE(rb[M_IOFF], 8 * (n + 1));
+    u64 *rec_off = (u64 *)rb[W_CNT].p, *ioff = (u64 *)rb[M_IOFF].p;
+    CK(cudaMemsetAsync(d_misc, 0, 8, ctx->stream));
+    size_t need = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, need, rec_off, rec_off, n + 1, ctx->stream);
+    ENSURE(ctx->scan_tmp, need);
+    k_mw_count<<<(unsigned)((n + 1 + 255) / 256), 256, 0, ctx->stream>>>(w, n, n_contigs, rec_off, ioff, d_misc);
+    CK(cub::DeviceScan::ExclusiveSum(ctx->scan_tmp.p, need, rec_off, rec_off, n + 1, ctx->stream));
+    CK(cub::DeviceScan::ExclusiveSum(ctx->scan_tmp.p, need, ioff, ioff, n + 1, ctx->stream));
+    unsigned long long h[3] = {0, 0, 0};
+    CK(cudaMemcpyAsync(&h[0], d_misc, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&h[1], rec_off + n, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&h[2], ioff + n, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->launches += 3;
+    CK(cudaGetLastError());
+    if ((rc = merge_bad(ctx, who, h[0])) != AVK_OK) return rc;
+    const u64 n_rec = h[1], info_bytes = h[2];
+    // the INFO texts, then the length pass and the scan of the line lengths (64-bit counts and offsets throughout)
+    ENSURE(rb[M_INFO], info_bytes);
+    u8 *info = (u8 *)rb[M_INFO].p;
+    if (info_bytes) {
+        k_mw_info<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(w, n, ioff, info);
+        ctx->launches += 1;
+    }
+    ENSURE(rb[W_LEN], 8 * (n_rec + 1));
+    ENSURE(rb[W_REG], 4 * n_rec);
+    u64 *off = (u64 *)rb[W_LEN].p;
+    u32 *reg = (u32 *)rb[W_REG].p;
+    need = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, need, off, off, n_rec + 1, ctx->stream);
+    ENSURE(ctx->scan_tmp, need);
+    k_mw_len<<<(unsigned)((n_rec + 1 + 255) / 256), 256, 0, ctx->stream>>>(w, n, n_rec, rec_off, ioff, reg, off);
+    CK(cub::DeviceScan::ExclusiveSum(ctx->scan_tmp.p, need, off, off, n_rec + 1, ctx->stream));
+    u64 body = 0;
+    CK(cudaMemcpyAsync(&body, off + n_rec, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->launches += 2;
+    CK(cudaGetLastError());
+    const u64 len = header_len + body;
+    if (bgzf_chunks(len) >= 0x7fffffffull) { ctx->err = std::string(who) + ": text too long for one call"; return AVK_ERR_INVALID; }
+    if (!out) { *out_len = bgzf_bound(len); return AVK_OK; }
+    // header + lines into rb[V_TEXT], then the compressor
+    ENSURE(rb[C_TEXT], len);
+    u8 *text = (u8 *)rb[C_TEXT].p;
+    if (header_len) CK(cudaMemcpyAsync(text, header, header_len, cudaMemcpyHostToDevice, ctx->stream));
+    if (n_rec) {
+        k_mw_write<<<(unsigned)((n_rec + 255) / 256), 256, 0, ctx->stream>>>(w, n_rec, reg, rec_off, ioff, info, off, header_len, text);
+        ctx->launches += 1;
+        CK(cudaGetLastError());
+    }
+    return bgzf_compress_device(ctx, len, eof != 0, out, cap, out_len);
+}
+
+extern "C" int avk_merge_regions_bgzf(avk_ctx *ctx, const char *const *contig_names, uint32_t n_contigs, int passing,
+                                      const uint64_t *region_id, int eof, uint8_t *out, uint64_t cap, uint64_t *out_len) {
+    static const char *who = "avk_merge_regions_bgzf";
+    if (!ctx) return AVK_ERR_INVALID;
+    if (!out_len) { ctx->err = std::string(who) + ": bad arguments"; return AVK_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->device));
+    MergeRecView w;
+    int rc = merge_view_device(ctx, who, contig_names, n_contigs, nullptr, region_id, true, w);
+    if (rc != AVK_OK) return rc;
+    DevBuf *rb = ctx->rb;
+    const u64 n = ctx->n_regions;
+    ENSURE(rb[W_MISC], 64);
+    unsigned long long *d_misc = (unsigned long long *)rb[W_MISC].p;
+    ENSURE(rb[W_LEN], 8 * (n + 1));
+    u64 *off = (u64 *)rb[W_LEN].p;
+    CK(cudaMemsetAsync(d_misc, 0, 8, ctx->stream));
+    size_t need = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, need, off, off, n + 1, ctx->stream);
+    ENSURE(ctx->scan_tmp, need);
+    k_mr_len<<<(unsigned)((n + 1 + 255) / 256), 256, 0, ctx->stream>>>(w, n, n_contigs, passing, off, d_misc);
+    CK(cub::DeviceScan::ExclusiveSum(ctx->scan_tmp.p, need, off, off, n + 1, ctx->stream));
+    unsigned long long h[2] = {0, 0};
+    CK(cudaMemcpyAsync(&h[0], d_misc, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&h[1], off + n, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->launches += 2;
+    CK(cudaGetLastError());
+    if ((rc = merge_bad(ctx, who, h[0])) != AVK_OK) return rc;
+    const u64 len = h[1];
+    if (bgzf_chunks(len) >= 0x7fffffffull) { ctx->err = std::string(who) + ": text too long for one call"; return AVK_ERR_INVALID; }
+    if (!out) { *out_len = bgzf_bound(len); return AVK_OK; }
+    ENSURE(rb[C_TEXT], len);
+    if (len) {
+        k_mr_write<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(w, n, off, (u8 *)rb[C_TEXT].p);
+        ctx->launches += 1;
+        CK(cudaGetLastError());
+    }
+    return bgzf_compress_device(ctx, len, eof != 0, out, cap, out_len);
+}
+
+// The summary's keys of the resident bin counted on the device: one key per variant (k_ms_keys), radix sort, run-length
+// encoding; only the distinct keys and their counts are copied to the host.
+extern "C" int avk_merge_summary_counts(avk_ctx *ctx, avk_merge_summary_row *rows, uint64_t cap, uint64_t *n_rows) {
+    static const char *who = "avk_merge_summary_counts";
+    if (!ctx) return AVK_ERR_INVALID;
+    if (!n_rows) { ctx->err = std::string(who) + ": bad arguments"; return AVK_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->device));
+    MergeRecView w;
+    int rc = merge_view_device(ctx, who, nullptr, 0, nullptr, nullptr, false, w);
+    if (rc != AVK_OK) return rc;
+    DevBuf *rb = ctx->rb;
+    const u64 n = ctx->n_regions, nv = ctx->n_variants;
+    *n_rows = 0;
+    if (nv == 0) return AVK_OK;
+    ENSURE(rb[W_MISC], 64);
+    unsigned long long *d_misc = (unsigned long long *)rb[W_MISC].p;     // [0] MW_BAD_* flags, [1] number of runs
+    ENSURE(rb[M_KEY], 8 * nv); ENSURE(rb[M_KEY_S], 8 * nv); ENSURE(rb[M_UNIQ], 8 * nv); ENSURE(rb[M_RUNS], 4 * nv);
+    u64 *key = (u64 *)rb[M_KEY].p, *key_s = (u64 *)rb[M_KEY_S].p, *uniq = (u64 *)rb[M_UNIQ].p;
+    u32 *runs = (u32 *)rb[M_RUNS].p;
+    u32 *n_runs = (u32 *)(d_misc + 1);
+    size_t tmp = 0, need = 0;
+    cub::DeviceRadixSort::SortKeys(nullptr, need, key, key_s, (int)nv, 0, 64, ctx->stream); tmp = std::max(tmp, need);
+    cub::DeviceRunLengthEncode::Encode(nullptr, need, key_s, uniq, runs, n_runs, (int)nv, ctx->stream); tmp = std::max(tmp, need);
+    ENSURE(ctx->scan_tmp, tmp);
+    CK(cudaMemsetAsync(d_misc, 0, 16, ctx->stream));
+    k_ms_keys<<<(unsigned)((nv + 255) / 256), 256, 0, ctx->stream>>>(w, n, ctx->v_base, nv, key, d_misc);
+    need = tmp; CK(cub::DeviceRadixSort::SortKeys(ctx->scan_tmp.p, need, key, key_s, (int)nv, 0, 64, ctx->stream));
+    need = tmp; CK(cub::DeviceRunLengthEncode::Encode(ctx->scan_tmp.p, need, key_s, uniq, runs, n_runs, (int)nv, ctx->stream));
+    unsigned long long h[2] = {0, 0};
+    CK(cudaMemcpyAsync(h, d_misc, 16, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->launches += 3;
+    CK(cudaGetLastError());
+    if ((rc = merge_bad(ctx, who, h[0])) != AVK_OK) return rc;
+    u64 m = (u32)h[1];
+    std::vector<u64> hk(m);
+    std::vector<u32> hc(m);
+    if (m) {
+        CK(cudaMemcpyAsync(hk.data(), uniq, 8 * m, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(hc.data(), runs, 4 * m, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    if (m && hk[m - 1] == ~0ull) --m;                             // the variants of unsolved regions
+    *n_rows = m;
+    if (!rows) return AVK_OK;
+    if (cap < m) { ctx->err = std::string(who) + ": row capacity too small"; return AVK_ERR_OOM; }
+    for (u64 i = 0; i < m; ++i) {
+        avk_merge_summary_row &o = rows[i];
+        const u64 k = hk[i];
+        o.indices = (u32)k; o.classification = (u8)(k >> 56); o.variant_type = (u8)(k >> 48); o.input = (u8)(k >> 40); o.pad = 0;
+        const bool pass = o.classification == AVK_MERGE_BASEPAIR_IDENTICAL || (o.indices >> o.input & 1u);
+        o.pass_variants = pass ? hc[i] : 0; o.fail_variants = pass ? 0 : hc[i];
+    }
+    return AVK_OK;
 }
 
 extern "C" int avk_vcf_parse_bgzf(avk_ctx *ctx, const uint8_t *gz, uint64_t gz_len, int verify_crc, const char *const *contig_names, uint32_t n_contigs,

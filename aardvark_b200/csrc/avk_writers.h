@@ -7,7 +7,8 @@
 //   * the three outputs of `aardvark merge` that are functions of the merge path's results (avk_merge_out):
 //     avk_merge_records_write (VariantMerger::write_variants, src/writers/variant_merger.rs:198-287: body lines of
 //     passing.vcf.gz), avk_merge_regions_write (write_region :294-309: regions.bed / failed_regions.bed) and
-//     avk_merge_summary_write (MergeSummaryWriter, src/writers/merge_summary.rs:56-112).
+//     avk_merge_summary_write (MergeSummaryWriter, src/writers/merge_summary.rs:56-112), whose ordering and formatting
+//     avk_merge_summary_rows_write shares for the per-key counts the device computes (avk_merge_summary_counts).
 // Plain C++17, no CUDA: the counters and labels were computed on the device, these functions only format them.
 #pragma once
 #include <charconv>
@@ -229,12 +230,15 @@ static inline std::string merge_regions_text(const avk_region_batch *b, const ch
 // MergeSummaryWriter (merge_summary.rs:56-112): pass / fail variant counts keyed by (MergeClassification, VariantType, vcf index)
 // in the derived Ord -- Different < NoConflict{indices} < MajorityAgree{indices} < ConflictSelection{index} <
 // BasepairIdentical, index lists compared lexicographically -- one row per key: merge_reason (Display: simplify() + "_i" per
-// index, merge_benchmark.rs:22-44), variant_type ({:?}), vcf_index, vcf_label, pass_variants, fail_variants
-static inline std::string merge_summary_text(const avk_region_batch *b, const char *const *labels, const MergeView &m, char delim, bool header) {
+// index, merge_benchmark.rs:22-44), variant_type ({:?}), vcf_index, vcf_label, pass_variants, fail_variants.
+// The counts of either source -- a batch and its result on the host, or the avk_merge_summary_row keys the device counted --
+// go into one ordered map, and one function writes it.
+typedef std::tuple<uint8_t, std::vector<uint8_t>, uint8_t, uint32_t> MergeSummaryKey;       // class, indices, variant type, vcf index
+typedef std::map<MergeSummaryKey, std::pair<uint64_t, uint64_t>> MergeSummaryCounts;       // key -> (pass, fail)
+
+static inline void merge_summary_count_batch(MergeSummaryCounts &counts, const avk_region_batch *b, const MergeView &m) {
     const avk_variant_table &t = b->variants;
     const uint64_t K = b->n_inputs;
-    typedef std::tuple<uint8_t, std::vector<uint8_t>, uint8_t, uint32_t> Key;       // class, indices, variant type, vcf index
-    std::map<Key, std::pair<uint64_t, uint64_t>> counts;
     for (uint64_t r = 0; r < b->n_regions; ++r) {
         if (!merge_solved(m, r)) continue;
         const uint8_t c = m.cls[r];
@@ -246,11 +250,24 @@ static inline std::string merge_summary_text(const avk_region_batch *b, const ch
             bool pass = c == AVK_MERGE_BASEPAIR_IDENTICAL;
             for (uint8_t i : ind) pass = pass || i == k;
             for (uint64_t v = b->var_off[r * K + k]; v < b->var_off[r * K + k + 1]; ++v) {
-                auto &e = counts[Key(c, ind, t.variant_type[v], (uint32_t)k)];
+                auto &e = counts[MergeSummaryKey(c, ind, t.variant_type[v], (uint32_t)k)];
                 if (pass) e.first += 1; else e.second += 1;
             }
         }
     }
+}
+// rows of one or several bins: the index list of a row is the ascending list of the bits of `indices`; rows that share a key
+// add up
+static inline void merge_summary_count_rows(MergeSummaryCounts &counts, const avk_merge_summary_row *rows, uint64_t n_rows) {
+    for (uint64_t i = 0; i < n_rows; ++i) {
+        const avk_merge_summary_row &w = rows[i];
+        std::vector<uint8_t> ind;
+        for (uint32_t k = 0; k < 32; ++k) if (w.indices >> k & 1u) ind.push_back((uint8_t)k);
+        auto &e = counts[MergeSummaryKey(w.classification, ind, w.variant_type, w.input)];
+        e.first += w.pass_variants; e.second += w.fail_variants;
+    }
+}
+static inline std::string merge_summary_format(const MergeSummaryCounts &counts, const char *const *labels, char delim, bool header) {
     std::string o;
     if (header && !counts.empty()) {        // (the csv crate writes the header with the first serialised row)
         const char *cols[6] = {"merge_reason", "variant_type", "vcf_index", "vcf_label", "pass_variants", "fail_variants"};
@@ -265,6 +282,11 @@ static inline std::string merge_summary_text(const avk_region_batch *b, const ch
         o += std::to_string(kv.second.first); o += delim; o += std::to_string(kv.second.second); o += '\n';
     }
     return o;
+}
+static inline std::string merge_summary_text(const avk_region_batch *b, const char *const *labels, const MergeView &m, char delim, bool header) {
+    MergeSummaryCounts counts;
+    merge_summary_count_batch(counts, b, m);
+    return merge_summary_format(counts, labels, delim, header);
 }
 
 }  // namespace avk_writers

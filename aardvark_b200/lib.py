@@ -96,6 +96,9 @@ def load():
     lib.avk_compare_upload.argtypes = [vp, C.POINTER(abi.RegionBatch)]
     lib.avk_compare_run_resident.argtypes = [vp, C.POINTER(abi.CompareCfg)]
     lib.avk_compare_download.argtypes = [vp, C.POINTER(abi.CompareOut)]
+    lib.avk_merge_upload_range.argtypes = [vp, C.POINTER(abi.RegionBatch), C.c_uint64, C.c_uint64]
+    lib.avk_merge_run_resident.argtypes = [vp, C.POINTER(abi.MergeCfg)]
+    lib.avk_merge_download.argtypes = [vp, C.POINTER(abi.MergeOut)]
     lib.avk_last_timings.argtypes = [vp, C.POINTER(C.c_float)]
     lib.avk_last_work.argtypes = [vp, C.POINTER(abi.WorkCounters)]
     lib.avk_int_peak.argtypes = [vp, C.POINTER(C.c_double)]
@@ -111,6 +114,8 @@ EXPORTED_SYMBOLS = [
     "avk_compare_result_device", "avk_set_stratifications", "avk_create_lane",
     "avk_merge_records_write", "avk_merge_regions_write", "avk_merge_summary_write", "avk_bgzf_inflate", "avk_vcf_parse_bgzf", "avk_bgzf_compress", "avk_spec_profile",
     "avk_compare_records_bgzf",
+    "avk_merge_upload_range", "avk_merge_run_resident", "avk_merge_download", "avk_merge_records_bgzf", "avk_merge_regions_bgzf",
+    "avk_merge_summary_counts", "avk_merge_summary_rows_write",
 ]
 
 
@@ -289,6 +294,25 @@ class Solver:
     def download(self, out: CompareOutputs):
         co = out.to_c()
         self._check(self._lib.avk_compare_download(self._ctx, C.byref(co)), "avk_compare_download")
+        return out
+
+    # -- resident merge: upload (or build_regions), solve, and write the outputs where the batch lies -------------------
+    def merge_upload(self, batch: RegionBatch, lo: int = None, hi: int = None):
+        """Regions [lo, hi) of `batch` (all by default) become the resident batch of a merge (avk_merge_upload_range)."""
+        cb = batch.to_c()
+        lo, hi = (0, batch.n_regions) if lo is None else (lo, hi)
+        self._check(self._lib.avk_merge_upload_range(self._ctx, C.byref(cb), lo, hi), "avk_merge_upload_range")
+
+    def merge_run_resident(self, cfg: MergeConfig = None):
+        """Solve the resident batch (merge_upload or build_regions); the result stays on the device for merge_download and the
+        device writers (writers.merge_records_bgzf / merge_regions_bgzf / merge_summary_rows)."""
+        cc = merge_cfg(cfg or MergeConfig())
+        self._check(self._lib.avk_merge_run_resident(self._ctx, C.byref(cc)), "avk_merge_run_resident")
+
+    def merge_download(self, out: MergeOutputs) -> MergeOutputs:
+        """The resident bin's merge result into out[lo:hi] (out is sized for the whole batch)."""
+        co = out.to_c()
+        self._check(self._lib.avk_merge_download(self._ctx, C.byref(co)), "avk_merge_download")
         return out
 
     def last_timings_ms(self):

@@ -26,6 +26,7 @@ def _bind():
     lib.avk_merge_records_write.argtypes = [C.POINTER(abi.RegionBatch), C.POINTER(abi.MergeOut), names, C.c_uint32, names, C.c_uint64, C.c_uint64] + t
     lib.avk_merge_regions_write.argtypes = [C.POINTER(abi.RegionBatch), C.POINTER(abi.MergeOut), names, C.c_uint32, C.c_int, C.c_uint64, C.c_uint64] + t
     lib.avk_merge_summary_write.argtypes = [C.POINTER(abi.RegionBatch), C.POINTER(abi.MergeOut), names, C.c_int, C.c_int] + t
+    lib.avk_merge_summary_rows_write.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, names, C.c_int, C.c_int] + t
     return lib
 
 
@@ -143,3 +144,75 @@ def vcf_records_bgzf(solver, side, contig_names, header: bytes = b"", region_ids
     out = np.empty(int(n.value), dtype=np.uint8)                 # an upper bound; pages past the compressed size are never touched
     solver._check(call(out.ctypes.data, out.size), "avk_compare_records_bgzf")
     return out[:int(n.value)].tobytes()
+
+
+def _bgzf_call(solver, what, call):
+    """size query (an upper bound), then the call into a buffer of that size"""
+    n = C.c_uint64(0)
+    solver._check(call(None, 0, C.byref(n)), what)
+    out = np.empty(int(n.value), dtype=np.uint8)                 # pages past the compressed size are never touched
+    solver._check(call(out.ctypes.data, out.size, C.byref(n)), what)
+    return out[:int(n.value)].tobytes()
+
+
+def _merge_bgzf_fns(lib):
+    names = C.POINTER(C.c_char_p)
+    t = [C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+    lib.avk_merge_records_bgzf.argtypes = [C.c_void_p, names, C.c_uint32, names, C.POINTER(C.c_uint64), C.c_char_p, C.c_uint64, C.c_int] + t
+    lib.avk_merge_regions_bgzf.argtypes = [C.c_void_p, names, C.c_uint32, C.c_int, C.POINTER(C.c_uint64), C.c_int] + t
+    lib.avk_merge_summary_counts.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+    return lib.avk_merge_records_bgzf, lib.avk_merge_regions_bgzf, lib.avk_merge_summary_counts
+
+
+def _c_names(names):
+    return (C.c_char_p * max(len(names), 1))(*[n if isinstance(n, bytes) else n.encode() for n in names])
+
+
+def merge_records_bgzf(solver, contig_names, input_labels, header: bytes = b"", region_ids=None, eof=True) -> bytes:
+    """avk_merge_records_bgzf: passing.vcf.gz of the solver's resident merge result, formatted and compressed on the device -- the
+    same bytes as bgzf_compress(solver, header + VariantMerger(...).passing_records(lo, hi)) over the resident bin.  region_ids:
+    the ids of the batch given to merge_upload() / merge_batch() (the whole batch's array), None after build_regions().
+    eof=False leaves out the EOF marker so that the next bin's file can be appended.  Labels are str or raw bytes."""
+    fn = _merge_bgzf_fns(solver._lib)[0]
+    names, labels = _c_names(contig_names), _c_names(input_labels)
+    rid = None if region_ids is None else np.ascontiguousarray(region_ids, dtype=np.uint64)
+    rid_p = abi.ptr(rid)
+    return _bgzf_call(solver, "avk_merge_records_bgzf", lambda buf, cap, n: fn(solver._ctx, names, len(contig_names), labels, rid_p, header, len(header),
+                                                                                1 if eof else 0, buf, cap, n))
+
+
+def merge_regions_bgzf(solver, contig_names, passing=True, region_ids=None, eof=True) -> bytes:
+    """avk_merge_regions_bgzf: regions.bed.gz (passing) / failed_regions.bed.gz of the resident merge result -- the same bytes as
+    bgzf_compress(solver, VariantMerger(...).regions_bed(passing, lo, hi)) over the resident bin."""
+    fn = _merge_bgzf_fns(solver._lib)[1]
+    names = _c_names(contig_names)
+    rid = None if region_ids is None else np.ascontiguousarray(region_ids, dtype=np.uint64)
+    rid_p = abi.ptr(rid)
+    return _bgzf_call(solver, "avk_merge_regions_bgzf", lambda buf, cap, n: fn(solver._ctx, names, len(contig_names), 1 if passing else 0, rid_p,
+                                                                                1 if eof else 0, buf, cap, n))
+
+
+# avk_merge_summary_row
+SUMMARY_ROW = np.dtype([("indices", np.uint32), ("classification", np.uint8), ("variant_type", np.uint8), ("input", np.uint8), ("pad", np.uint8),
+                        ("pass_variants", np.uint64), ("fail_variants", np.uint64)], align=True)
+
+
+def merge_summary_rows(solver) -> np.ndarray:
+    """avk_merge_summary_counts: the merge summary's per-key variant counts of the resident bin, counted on the device (a
+    SUMMARY_ROW array in no particular order).  Rows of several bins or GPUs are simply concatenated for merge_summary_text."""
+    fn = _merge_bgzf_fns(solver._lib)[2]
+    n = C.c_uint64(0)
+    solver._check(fn(solver._ctx, None, 0, C.byref(n)), "avk_merge_summary_counts")
+    rows = np.zeros(max(int(n.value), 1), dtype=SUMMARY_ROW)
+    solver._check(fn(solver._ctx, rows.ctypes.data, rows.size, C.byref(n)), "avk_merge_summary_counts")
+    return rows[:int(n.value)]
+
+
+def merge_summary_text(rows, n_inputs, labels, csv=False, header=True) -> str:
+    """avk_merge_summary_rows_write (host): the merge summary of the rows -- the text VariantMerger.summary_text gives over the
+    whole batch.  Rows that share a key add up."""
+    lib = _bind()
+    rows = np.ascontiguousarray(rows, dtype=SUMMARY_ROW)
+    lab = _c_names(labels)
+    return _text(lambda buf, cap, n: lib.avk_merge_summary_rows_write(rows.ctypes.data if rows.size else None, rows.size, n_inputs, lab,
+                                                                      1 if csv else 0, 1 if header else 0, buf, cap, n))

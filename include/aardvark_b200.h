@@ -442,6 +442,48 @@ int avk_merge_regions_write(const avk_region_batch *batch, const avk_merge_out *
 int avk_merge_summary_write(const avk_region_batch *batch, const avk_merge_out *result, const char *const *input_labels, int csv, int header,
                             char *buf, uint64_t cap, uint64_t *len);
 
+/* ---- resident merge: the batch stays on the device between the merge and its outputs (the merge chain K BGZF VCFs ->
+ * avk_vcf_parse_bgzf -> avk_build_regions_bed -> avk_merge_run_resident -> the writers below never sends the batch or the
+ * result to the host).
+ * avk_merge_upload_range: regions [lo, hi) of a host batch (1 <= n_inputs <= 32) become the resident batch.
+ * avk_merge_run_resident: solves the resident batch (from avk_merge_upload_range or avk_build_regions[_bed]); the merge
+ *   result stays on the device.  It overwrites the status array a compare result uses: after it avk_compare_download,
+ *   avk_compare_result_device and avk_compare_records_bgzf are refused, and a compare run (or any upload, build,
+ *   avk_set_reference or avk_wfa_ed_batch) in turn drops the merge result.  avk_merge_batch leaves its result resident as
+ *   well, and so does every context of avk_merge_batch_multi for its own bin.
+ * avk_merge_download: status / classification / n_indices / indices of the resident bin into out->...[lo, hi) (out->status
+ *   required, the others may be NULL).
+ * Every merge call below fails with AVK_ERR_INVALID (and a message) when no merge result is resident; the context stays usable. */
+int avk_merge_upload_range(avk_ctx *ctx, const avk_region_batch *batch, uint64_t lo, uint64_t hi);
+int avk_merge_run_resident(avk_ctx *ctx, const avk_merge_cfg *cfg);
+int avk_merge_download(avk_ctx *ctx, avk_merge_out *out);
+/* passing.vcf.gz and regions.bed.gz / failed_regions.bed.gz of the resident merge result, formatted and BGZF-compressed on the
+ * device: out = byte for byte avk_bgzf_compress(header || avk_merge_records_write(batch, result, contig_names, n_contigs,
+ * input_labels, lo, lo + n)), resp. avk_bgzf_compress(avk_merge_regions_write(batch, result, contig_names, n_contigs, passing,
+ * lo, lo + n)), for the resident bin [lo, lo + n).  region_id, eof, out == NULL (an upper bound of the size) and cap < size
+ * (AVK_ERR_OOM with *out_len = the exact size) behave as in avk_compare_records_bgzf.  A region whose contig is >= n_contigs,
+ * a null contig name or a null label (input_labels has n_inputs entries) fails the call with AVK_ERR_INVALID. */
+int avk_merge_records_bgzf(avk_ctx *ctx, const char *const *contig_names, uint32_t n_contigs, const char *const *input_labels,
+                           const uint64_t *region_id, const uint8_t *header, uint64_t header_len, int eof,
+                           uint8_t *out, uint64_t cap, uint64_t *out_len);
+int avk_merge_regions_bgzf(avk_ctx *ctx, const char *const *contig_names, uint32_t n_contigs, int passing,
+                           const uint64_t *region_id, int eof, uint8_t *out, uint64_t cap, uint64_t *out_len);
+/* The merge summary without the batch on the host.  A row counts the variants of one key (classification, index list,
+ * variant type, input) over the solved regions of the resident bin; the index list is a bit mask (bit k <=> input k; for
+ * conflict selection the selected input), and a key's variants all pass or all fail.  avk_merge_summary_counts: the keys are
+ * counted on the device (sort + run-length encoding), only the distinct ones are copied; rows == NULL: *n_rows = the number
+ * of rows; cap < that number: AVK_ERR_OOM with *n_rows set.  Rows come in no particular order.
+ * avk_merge_summary_rows_write (host only): rows of one or several bins / GPUs, simply concatenated (rows that share a key
+ * add up) -> the text avk_merge_summary_write gives over the whole batch, in the same order and csv quoting. */
+typedef struct avk_merge_summary_row {
+    uint32_t indices;
+    uint8_t classification, variant_type, input, pad;
+    uint64_t pass_variants, fail_variants;
+} avk_merge_summary_row;
+int avk_merge_summary_counts(avk_ctx *ctx, avk_merge_summary_row *rows, uint64_t cap, uint64_t *n_rows);
+int avk_merge_summary_rows_write(const avk_merge_summary_row *rows, uint64_t n_rows, uint32_t n_inputs, const char *const *input_labels,
+                                 int csv, int header, char *buf, uint64_t cap, uint64_t *len);
+
 int avk_compare_upload(avk_ctx *ctx, const avk_region_batch *batch);
 int avk_compare_upload_range(avk_ctx *ctx, const avk_region_batch *batch, uint64_t lo, uint64_t hi);
 int avk_compare_run_resident(avk_ctx *ctx, const avk_compare_cfg *cfg);
