@@ -28,6 +28,7 @@ N_GROUPS = 1 + N_VARIANT_TYPES
 
 ST_OK, ST_BAD_ZYGOSITY, ST_NO_RESULT, ST_TRUTH_FP, ST_TP_UNDERFLOW, ST_BAD_INPUT, ST_WORKSPACE, ST_TIMEOUT = range(8)
 CMP_KEEP_REGION_ROWS = 1
+CMP_KEEP_SEQUENCES = 2
 
 AVK_OK, AVK_ERR_INVALID, AVK_ERR_CUDA, AVK_ERR_NO_REFERENCE, AVK_ERR_OOM = 0, -1, -2, -3, -4
 

@@ -1271,6 +1271,7 @@ struct avk_ctx {
     bool have_batch = false;
     bool ids_resident = false;      // the resident batch was built on the device (avk_build_regions*): its region ids are in `region_id`
     bool have_result = false, result_has_rows = false;
+    bool result_has_seq = false;    // the last compare pass filled the sequence bundle (seq_off / seq_len / seq_pool, offsets biased by seq_base)
     bool have_merge = false;        // the last pass was a merge: its result (status, m_cls, m_nidx, m_idx) is resident; cleared with have_result
     bool result_has_contain = false;   // the last pass filled st_mask (a resident run never computes containment)
     u64 lo = 0, n_regions = 0, v_base = 0, n_variants = 0, p_base = 0, pool_bytes = 0;
@@ -1529,7 +1530,7 @@ extern "C" int avk_set_reference(avk_ctx *ctx, uint32_t n_contigs, const uint8_t
     UPLOAD(ctx->d_contig_ptr, ptrs.data(), sizeof(u8 *) * n_contigs);
     UPLOAD(ctx->d_contig_len, lens, sizeof(u64) * n_contigs);
     CK(cudaStreamSynchronize(ctx->stream));
-    ctx->have_result = ctx->have_merge = false;
+    ctx->have_result = ctx->have_merge = ctx->result_has_seq = false;
     return AVK_OK;
 }
 
@@ -1648,7 +1649,7 @@ static int upload_batch(avk_ctx *ctx, const avk_region_batch *b, BinScan &sc) {
     if (ref_of(ctx)->contig_bufs.empty()) { ctx->err = "avk_set_reference has not been called"; return AVK_ERR_NO_REFERENCE; }
     const u64 lo = sc.lo, n = sc.hi - sc.lo, K = b->n_inputs, v0 = sc.v0, nv = sc.v1 - sc.v0;
     const avk_variant_table &t = b->variants;
-    ctx->have_batch = false; ctx->have_result = ctx->have_merge = false; ctx->ids_resident = false;
+    ctx->have_batch = false; ctx->have_result = ctx->have_merge = ctx->result_has_seq = false; ctx->ids_resident = false;
     UPLOAD(ctx->contig, b->contig + lo, 4 * n);
     UPLOAD(ctx->start, b->start + lo, 4 * n);
     UPLOAD(ctx->end, b->end + lo, 4 * n);
@@ -2097,7 +2098,7 @@ static int compare_launch(avk_ctx *ctx, const avk_compare_cfg *cfg, bool want_se
     R.strat_idx = (strata && !strat_dev) ? biased<const u32>(ctx->strat_idx, ctx->strat_base) : nullptr;
     R.strat_mask = (strata && strat_dev) ? (const u64 *)ctx->st_mask.p : nullptr;
     R.want_contain = strat_dev || want_contain;
-    ctx->have_result = ctx->have_merge = false;
+    ctx->have_result = ctx->have_merge = ctx->result_has_seq = false;
 
     CK(cudaEventRecord(ctx->ev[0], ctx->stream));
     int rc = run_alt_ed(ctx, R.db);
@@ -2119,6 +2120,7 @@ static int compare_launch(avk_ctx *ctx, const avk_compare_cfg *cfg, bool want_se
     if (rc != AVK_OK) return rc;
     CK(cudaEventRecord(ctx->ev[4], ctx->stream));
     ctx->result_has_rows = rows;
+    ctx->result_has_seq = want_seq && cfg->enable_sequences;   // (the kernels emit the bundle only under enable_sequences)
     ctx->result_has_contain = R.want_contain;
     return queue_counter_copies(ctx);
 }
@@ -2533,7 +2535,7 @@ static int compare_lanes(avk_ctx *ctx, const avk_region_batch *batch, const avk_
     int rc = ensure_lanes(ctx, n);
     if (rc != AVK_OK) return rc;
     rc = compare_bins_concurrent(ctx->lanes.data(), (uint32_t)n, batch, cfg, out);
-    ctx->have_batch = ctx->have_result = ctx->have_merge = false;   // the owner holds one bin only: nothing "resident" to re-run or download
+    ctx->have_batch = ctx->have_result = ctx->have_merge = ctx->result_has_seq = false;   // the owner holds one bin only: nothing "resident" to re-run or download
     // the owner's timings describe the call: the longest device pass of the lanes
     for (int i = 1; i < n; ++i) if (ctx->lanes[i]->last_ms[4] > ctx->last_ms[4]) for (int k = 0; k < 5; ++k) ctx->last_ms[k] = ctx->lanes[i]->last_ms[k];
     return rc;
@@ -2701,7 +2703,7 @@ static int build_regions_impl(avk_ctx *ctx, const avk_callsets *in, const uint32
         }
     }
     if (sum_alle >= 0xffffffffull) { ctx->err = "avk_build_regions: allele bytes exceed 4 GiB"; return AVK_ERR_INVALID; }
-    ctx->have_batch = false; ctx->have_result = ctx->have_merge = false; ctx->ids_resident = false;
+    ctx->have_batch = false; ctx->have_result = ctx->have_merge = ctx->result_has_seq = false; ctx->ids_resident = false;
     ctx->lo = 0; ctx->v_base = 0; ctx->p_base = 0; ctx->pool_bytes = 0;
     *n_regions_out = 0; *n_variants_out = 0;
     if (nv == 0) { ctx->n_regions = 0; ctx->n_variants = 0; ctx->n_inputs = (u32)K; ctx->max_allele = 1; ctx->pool_len = 0; ctx->have_batch = ctx->ids_resident = true; ENSURE(ctx->var_off, 8); CK(cudaMemsetAsync(ctx->var_off.p, 0, 8, ctx->stream)); return AVK_OK; }
@@ -2810,12 +2812,53 @@ extern "C" int avk_compare_upload(avk_ctx *ctx, const avk_region_batch *batch) {
     return avk_compare_upload_range(ctx, batch, 0, batch->n_regions);
 }
 
+// AVK_CMP_KEEP_SEQUENCES: the layout avk_compare_seq_offsets gives the resident bin (offsets from 0), built on the device --
+// per region the sizes {win, win + alt0, win + alt0, win + alt1, win + alt1} (k_seq_sizes), an exclusive scan into seq_off,
+// and the pool sized from the scan's total
+__global__ void __launch_bounds__(256) k_seq_sizes(DevBatch b, u64 n, u64 *sizes) {
+    const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r > n) return;
+    if (r == n) { sizes[n * 5] = 0; return; }
+    const u64 win = b.end[r] > b.start[r] ? b.end[r] - b.start[r] : 0;
+    u64 alt[2] = {0, 0};
+    for (int k = 0; k < 2; ++k)
+        for (u64 v = b.var_off[r * 2 + k]; v < b.var_off[r * 2 + k + 1]; ++v) alt[k] += b.l1[v];
+    u64 *o = sizes + r * 5;
+    o[0] = win; o[1] = o[2] = win + alt[0]; o[3] = o[4] = win + alt[1];
+}
+static int resident_seq_layout(avk_ctx *ctx) {
+    const u64 n = ctx->n_regions, m = n * 5 + 1;
+    ctx->result_has_seq = false;                                  // the buffers below are overwritten from here on
+    ENSURE(ctx->seq_off, 8 * m);
+    ENSURE(ctx->seq_len, 4 * 5 * n + 4);
+    u64 *off = (u64 *)ctx->seq_off.p;
+    size_t need = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, need, off, off, m, ctx->stream);
+    ENSURE(ctx->scan_tmp, need);
+    k_seq_sizes<<<(unsigned)((n + 1 + 255) / 256), 256, 0, ctx->stream>>>(dev_batch(ctx), n, off);
+    CK(cub::DeviceScan::ExclusiveSum(ctx->scan_tmp.p, need, off, off, m, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->h_pin, off + n * 5, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->launches += 2;
+    CK(cudaGetLastError());
+    u64 pool = 0;
+    memcpy(&pool, ctx->h_pin, 8);
+    ENSURE(ctx->seq_pool, pool);
+    CK(cudaMemsetAsync(ctx->seq_len.p, 0, 4 * 5 * n + 4, ctx->stream));
+    ctx->seq_base = 0;
+    return AVK_OK;
+}
+
 extern "C" int avk_compare_run_resident(avk_ctx *ctx, const avk_compare_cfg *cfg) {
     if (!ctx) return AVK_ERR_INVALID;
     if (!cfg || !ctx->have_batch || ctx->n_inputs != 2) { ctx->err = "no resident compare batch"; return AVK_ERR_INVALID; }
+    const bool keep_seq = (cfg->flags & AVK_CMP_KEEP_SEQUENCES) != 0;
+    if (keep_seq && !cfg->enable_sequences) { ctx->err = "AVK_CMP_KEEP_SEQUENCES needs enable_sequences"; return AVK_ERR_INVALID; }
     CK(cudaSetDevice(ctx->device));
     CompareRun R;
-    int rc = compare_launch(ctx, cfg, false, (cfg->flags & AVK_CMP_KEEP_REGION_ROWS) != 0, false, 0, false, false, R);
+    int rc = keep_seq ? resident_seq_layout(ctx) : AVK_OK;
+    if (rc != AVK_OK) return rc;
+    rc = compare_launch(ctx, cfg, keep_seq, (cfg->flags & AVK_CMP_KEEP_REGION_ROWS) != 0, false, 0, false, false, R);
     if (rc != AVK_OK) return rc;
     rc = compare_finish(ctx, R, nullptr);
     if (rc != AVK_OK) return rc;
@@ -2899,7 +2942,7 @@ extern "C" int avk_last_work(avk_ctx *ctx, avk_work_counters *out) {
 static int merge_launch(avk_ctx *ctx, const avk_merge_cfg *cfg) {
     const u64 n = ctx->n_regions;
     const u32 K = ctx->n_inputs;
-    ctx->have_result = ctx->have_merge = false;                 // the pass overwrites `status`, which a compare result owns too
+    ctx->have_result = ctx->have_merge = ctx->result_has_seq = false;                 // the pass overwrites `status`, which a compare result owns too
     ENSURE(ctx->status, 4 * n); ENSURE(ctx->m_cls, n); ENSURE(ctx->m_nidx, n); ENSURE(ctx->m_idx, n * K);
     ENSURE(ctx->counters, 64); ENSURE(ctx->work_ctr, 64);
     CK(cudaMemsetAsync(ctx->work_ctr.p, 0, 64, ctx->stream));
@@ -3096,7 +3139,7 @@ extern "C" int avk_wfa_ed_batch(avk_ctx *ctx, uint64_t n_pairs, const uint8_t *p
     CK(cudaEventRecord(ctx->ev[2], ctx->stream));
     CK(cudaEventRecord(ctx->ev[3], ctx->stream));
     CK(cudaEventRecord(ctx->ev[4], ctx->stream));
-    ctx->have_result = ctx->have_merge = false;
+    ctx->have_result = ctx->have_merge = ctx->result_has_seq = false;
     CK(cudaMemcpyAsync(ed_out, ctx->pair_ed.p, 4 * n_pairs, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(ctx->h_pin + 128, ctx->work_ctr.p, 40, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaEventRecord(ctx->ev_done, ctx->stream));
@@ -3140,6 +3183,31 @@ extern "C" int avk_vcf_records_write(const avk_region_batch *batch, uint32_t sid
     if (!batch || !contig_names || !var_class || !var_expected || !var_observed || side >= batch->n_inputs || lo > hi || hi > batch->n_regions) return AVK_ERR_INVALID;
     for (uint64_t r = lo; r < hi; ++r) if (batch->contig[r] >= n_contigs) return AVK_ERR_INVALID;
     return copy_text(avk_writers::vcf_records_text(batch, side, contig_names, var_class, var_expected, var_observed, lo, hi), buf, cap, len);
+}
+
+// the argument checks both debug writers share, host and device: names present and printable without quoting
+static bool debug_names_ok(const char *const *contig_names, uint32_t n_contigs) {
+    if (!contig_names && n_contigs) return false;
+    for (uint32_t c = 0; c < n_contigs; ++c) if (!contig_names[c] || !avk_writers::plain_name(contig_names[c])) return false;
+    return true;
+}
+static bool debug_range_ok(const avk_region_batch *batch, const int32_t *status, uint32_t n_contigs, uint64_t lo, uint64_t hi) {
+    if (!batch || !status || lo > hi || hi > batch->n_regions) return false;
+    for (uint64_t r = lo; r < hi; ++r) if (batch->contig[r] >= n_contigs) return false;
+    return true;
+}
+extern "C" int avk_region_summary_write(const avk_region_batch *batch, const int32_t *status, const uint64_t *region_metrics,
+                                        const char *const *contig_names, uint32_t n_contigs, const uint8_t *metrics, uint32_t n_metrics, int header,
+                                        uint64_t lo, uint64_t hi, char *buf, uint64_t cap, uint64_t *len) {
+    if (!region_metrics || (!metrics && n_metrics) || !debug_names_ok(contig_names, n_contigs) || !debug_range_ok(batch, status, n_contigs, lo, hi)) return AVK_ERR_INVALID;
+    for (uint32_t q = 0; q < n_metrics; ++q) if (metrics[q] > 4) return AVK_ERR_INVALID;
+    return copy_text(avk_writers::region_summary_text(batch, status, region_metrics, contig_names, metrics, n_metrics, header != 0, lo, hi), buf, cap, len);
+}
+extern "C" int avk_region_sequences_write(const avk_region_batch *batch, const int32_t *status, const uint64_t *seq_off, const uint32_t *seq_len,
+                                          const uint8_t *seq_pool, const char *const *contig_names, uint32_t n_contigs, int header,
+                                          uint64_t lo, uint64_t hi, char *buf, uint64_t cap, uint64_t *len) {
+    if (!seq_off || !seq_len || !seq_pool || !debug_names_ok(contig_names, n_contigs) || !debug_range_ok(batch, status, n_contigs, lo, hi)) return AVK_ERR_INVALID;
+    return copy_text(avk_writers::region_sequences_text(batch, status, seq_off, seq_len, seq_pool, contig_names, header != 0, lo, hi), buf, cap, len);
 }
 
 static int merge_view(const avk_region_batch *batch, const avk_merge_out *res, uint32_t n_contigs, bool need_contigs, avk_writers::MergeView &m) {
@@ -3519,6 +3587,44 @@ extern "C" int avk_bgzf_compress(avk_ctx *ctx, const uint8_t *text, uint64_t len
 // are copied by the whole warp, so an SV allele (or one of the 16 MiB scan_bin admits) does not hold up its warp's other lines.
 enum { W_CNT = V_VOFF, W_LEN = V_BOFF, W_NAMES = V_NAMES, W_MISC = V_MISC, W_REG = V_C, W_RID = V_POS };   // off the compressor's slots
 enum { RW_LONG = 32 };
+// The contig names (and, for the merge records, the input labels) of a device writer, packed into rb[W_NAMES]: the
+// [n_contigs + 1] name offsets, the [n_labels + 1] label offsets (from the first label), then the names and the labels.
+// plain: refuse a name the debug writers would have to quote (avk_writers.h::plain_name).
+struct NameTable {
+    const u64 *name_off, *label_off;
+    const char *names, *labels;
+};
+static int upload_names(avk_ctx *ctx, const char *who, const char *const *contig_names, u32 n_contigs, const char *const *labels, u64 n_labels,
+                        bool plain, NameTable &t) {
+    std::vector<u64> tab(n_contigs + 1 + (labels ? n_labels + 1 : 0), 0);
+    std::string packed;
+    for (u32 c = 0; c < n_contigs; ++c) {
+        if (!contig_names[c]) { ctx->err = std::string(who) + ": null contig name"; return AVK_ERR_INVALID; }
+        if (plain && !avk_writers::plain_name(contig_names[c])) {
+            ctx->err = std::string(who) + ": a contig name contains a tab, '\"', CR or LF";
+            return AVK_ERR_INVALID;
+        }
+        packed += contig_names[c];
+        tab[c + 1] = packed.size();
+    }
+    const u64 names_len = packed.size();
+    if (labels) {
+        u64 *lt = tab.data() + n_contigs + 1;
+        for (u64 k = 0; k < n_labels; ++k) {
+            if (!labels[k]) { ctx->err = std::string(who) + ": null input label"; return AVK_ERR_INVALID; }
+            packed += labels[k];
+            lt[k + 1] = packed.size() - names_len;
+        }
+    }
+    DevBuf *rb = ctx->rb;
+    const size_t tab_bytes = 8 * tab.size();
+    ENSURE(rb[W_NAMES], tab_bytes + packed.size());
+    CK(cudaMemcpyAsync(rb[W_NAMES].p, tab.data(), tab_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    if (!packed.empty()) CK(cudaMemcpyAsync((u8 *)rb[W_NAMES].p + tab_bytes, packed.data(), packed.size(), cudaMemcpyHostToDevice, ctx->stream));
+    t.name_off = (const u64 *)rb[W_NAMES].p; t.label_off = t.name_off + n_contigs + 1;
+    t.names = (const char *)rb[W_NAMES].p + tab_bytes; t.labels = t.names + names_len;
+    return AVK_OK;
+}
 struct RecView {
     const u64 *var_off, *rid;
     const u32 *contig, *pos, *aoff, *l0, *l1;
@@ -3638,22 +3744,14 @@ extern "C" int avk_compare_records_bgzf(avk_ctx *ctx, uint32_t side, const char 
     CK(cudaSetDevice(ctx->device));
     DevBuf *rb = ctx->rb;
     const u64 n = ctx->n_regions, K = ctx->n_inputs;
-    std::vector<u64> name_tab(n_contigs + 1, 0);
-    std::string packed;
-    for (u32 c = 0; c < n_contigs; ++c) {
-        if (!contig_names[c]) { ctx->err = "avk_compare_records_bgzf: null contig name"; return AVK_ERR_INVALID; }
-        packed += contig_names[c];
-        name_tab[c + 1] = packed.size();
-    }
-    const size_t tab_bytes = 8 * name_tab.size();
-    ENSURE(rb[W_NAMES], tab_bytes + packed.size());
-    CK(cudaMemcpyAsync(rb[W_NAMES].p, name_tab.data(), tab_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    if (!packed.empty()) CK(cudaMemcpyAsync((u8 *)rb[W_NAMES].p + tab_bytes, packed.data(), packed.size(), cudaMemcpyHostToDevice, ctx->stream));
+    NameTable nt;
+    int rc = upload_names(ctx, "avk_compare_records_bgzf", contig_names, n_contigs, nullptr, 0, false, nt);
+    if (rc != AVK_OK) return rc;
     const DevBatch db = dev_batch(ctx);
     RecView w;
     w.var_off = db.var_off; w.contig = db.contig; w.pos = db.pos; w.aoff = db.aoff; w.l0 = db.l0; w.l1 = db.l1; w.zyg = db.zyg; w.pool = db.pool;
     w.cls = biased<const u8>(ctx->vcls, ctx->v_base); w.exp = biased<const u8>(ctx->vexp, ctx->v_base); w.obs = biased<const u8>(ctx->vobs, ctx->v_base);
-    w.name_off = (const u64 *)rb[W_NAMES].p; w.names = (const char *)rb[W_NAMES].p + tab_bytes;
+    w.name_off = nt.name_off; w.names = nt.names;
     w.K = (u32)K; w.side = side;
     if (region_id) {                                              // the caller's ids of the resident bin [lo, lo + n)
         UPLOAD(rb[W_RID], region_id + ctx->lo, 8 * n);
@@ -3708,6 +3806,276 @@ extern "C" int avk_compare_records_bgzf(avk_ctx *ctx, uint32_t side, const char 
         CK(cudaGetLastError());
     }
     return bgzf_compress_device(ctx, len, eof != 0, out, cap, out_len);
+}
+
+// ---- the debug folder of the resident compare, formatted on the device (avk_writers.h::region_summary_text and
+// region_sequences_text) ----------------------------------------------------------------------------------------------------
+// region_summary.tsv: count pass (one thread per region: n_metrics lines when solved, contig check) -> 64-bit scan -> length
+// pass (one thread per line; a line is a (solved region, metric) pair) -> scan -> write pass -> bgzf_compress_device.
+// region_sequences.tsv: length pass (one thread per region) -> scan -> write pass.  Strings longer than RW_LONG bytes are
+// copied by the whole warp: SV windows reach 64 kbp and more, so one line can be longer than a BGZF member.
+struct RegionView {
+    const u64 *rid;
+    const u32 *contig, *start, *end;
+    const int *status;
+    const u64 *rows;                     // [n][RED_COLS] per-region metric rows
+    const u64 *seq_off;                  // [n * 5 + 1], values biased by seq_base
+    const u32 *seq_len;                  // [n * 5]
+    const u8 *seq_pool;                  // biased by seq_base: string s of region r starts at seq_pool + seq_off[r * 5 + s]
+    const u8 *metrics;
+    u32 n_metrics;
+    NameTable nt;
+};
+__device__ __forceinline__ u32 rv_name_len(const RegionView &w, u32 c) { return (u32)(w.nt.name_off[c + 1] - w.nt.name_off[c]); }
+// "region_id \t chrom:start+1-end" (avk_writers.h::region_key)
+__device__ __forceinline__ u64 rv_key_len(const RegionView &w, u64 r) {
+    return rw_digits(w.rid[r]) + 1 + rv_name_len(w, w.contig[r]) + 1 + rw_digits((u64)w.start[r] + 1) + 1 + rw_digits(w.end[r]);
+}
+__device__ __forceinline__ u8 *rv_put_key(const RegionView &w, u64 r, u8 *o) {
+    o = rw_put_u64(o, w.rid[r], rw_digits(w.rid[r])); *o++ = '\t';
+    const u32 c = w.contig[r];
+    o = rw_put_str(o, w.nt.names + w.nt.name_off[c], rv_name_len(w, c)); *o++ = ':';
+    const u64 s = (u64)w.start[r] + 1;
+    o = rw_put_u64(o, s, rw_digits(s)); *o++ = '-';
+    return rw_put_u64(o, w.end[r], rw_digits(w.end[r]));
+}
+// avk_writers.h::METRIC_NAMES / METRIC_COL
+__device__ __forceinline__ const char *rs_metric(u32 m, u32 &n, u32 &col) {
+    switch (m) {
+        case 0: n = 2; col = AVK_M_GT; return "GT";
+        case 1: n = 3; col = AVK_M_HAP; return "HAP";
+        case 2: n = 12; col = AVK_M_WEIGHTED_HAP; return "WEIGHTED_HAP";
+        case 3: n = 8; col = AVK_M_BASEPAIR; return "BASEPAIR";
+        default: n = 9; col = AVK_M_RECORD_BP; return "RECORD_BP";
+    }
+}
+__global__ void __launch_bounds__(256) k_rs_count(RegionView w, u64 n, u32 n_contigs, u64 *cnt, unsigned long long *bad) {
+    const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r > n) return;
+    if (r == n) { cnt[n] = 0; return; }
+    cnt[r] = w.status[r] == 0 ? w.n_metrics : 0;
+    if (w.contig[r] >= n_contigs) atomicMax(bad, 1ull);
+}
+__global__ void __launch_bounds__(256) k_rs_len(RegionView w, u64 n, u64 n_lines, const u64 *line_off, u32 *reg, u64 *len) {
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i > n_lines) return;
+    if (i == n_lines) { len[n_lines] = 0; return; }
+    const u64 r = rw_region(line_off, n, i);
+    u32 nm, col;
+    const u32 m = w.metrics[i - line_off[r]];
+    rs_metric(m, nm, col);
+    const u64 *row = w.rows + r * RED_COLS;                       // the joint group
+    u64 l = rv_key_len(w, r) + 1 + nm + 4 + rw_digits(row[col]) + rw_digits(row[col + 1]) + rw_digits(row[col + 2]) + rw_digits(row[col + 3]) + 3;
+    if (m == 0) l += rw_digits(row[AVK_M_GT_TRUTH_FN_GT]) + rw_digits(row[AVK_M_GT_QUERY_FP_GT]);
+    reg[i] = (u32)r;
+    len[i] = l;
+}
+// off = exclusive scan of the line lengths; line i starts at text + base + off[i]
+__global__ void __launch_bounds__(256) k_rs_write(RegionView w, u64 n_lines, const u32 *reg, const u64 *line_off, const u64 *off, u64 base, u8 *text) {
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_lines) return;
+    const u64 r = reg[i];
+    u32 nm, col;
+    const u32 m = w.metrics[i - line_off[r]];
+    const char *name = rs_metric(m, nm, col);
+    const u64 *row = w.rows + r * RED_COLS;
+    u8 *o = rv_put_key(w, r, text + base + off[i]);
+    *o++ = '\t';
+    o = rw_put_str(o, name, nm);
+    for (u32 k = 0; k < 4; ++k) { *o++ = '\t'; o = rw_put_u64(o, row[col + k], rw_digits(row[col + k])); }
+    *o++ = '\t';
+    if (m == 0) o = rw_put_u64(o, row[AVK_M_GT_TRUTH_FN_GT], rw_digits(row[AVK_M_GT_TRUTH_FN_GT]));
+    *o++ = '\t';
+    if (m == 0) o = rw_put_u64(o, row[AVK_M_GT_QUERY_FP_GT], rw_digits(row[AVK_M_GT_QUERY_FP_GT]));
+    *o = '\n';
+}
+__global__ void __launch_bounds__(256) k_rq_len(RegionView w, u64 n, u32 n_contigs, u64 *len, unsigned long long *bad) {
+    const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r > n) return;
+    if (r == n) { len[n] = 0; return; }
+    if (w.contig[r] >= n_contigs) { atomicMax(bad, 1ull); len[r] = 0; return; }
+    u64 l = 0;
+    if (w.status[r] == 0) {
+        l = rv_key_len(w, r) + 5 + 1;
+        for (int s = 0; s < 5; ++s) l += w.seq_len[r * 5 + s];
+    }
+    len[r] = l;
+}
+__global__ void __launch_bounds__(256) k_rq_write(RegionView w, u64 n, const u64 *off, u64 base, u8 *text) {
+    const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool act = r < n && off[r + 1] > off[r];
+    u64 at[5] = {0, 0, 0, 0, 0};
+    bool any_long = false;
+    if (act) {
+        u8 *o = rv_put_key(w, r, text + base + off[r]);
+#pragma unroll
+        for (int s = 0; s < 5; ++s) {
+            *o++ = '\t';
+            const u32 l = w.seq_len[r * 5 + s];
+            at[s] = (u64)(o - text);
+            if (l <= RW_LONG) rw_put_str(o, (const char *)w.seq_pool + w.seq_off[r * 5 + s], l);
+            else any_long = true;
+            o += l;
+        }
+        *o = '\n';
+    }
+    const int lane = lane_id();
+    for (u32 m = __ballot_sync(AVK_FULL, any_long); m; m &= m - 1) {
+        const int src_lane = __ffs(m) - 1;
+        const u64 rr = __shfl_sync(AVK_FULL, r, src_lane);
+#pragma unroll
+        for (int s = 0; s < 5; ++s) {
+            const u64 d = __shfl_sync(AVK_FULL, at[s], src_lane);
+            const u32 l = w.seq_len[rr * 5 + s];
+            if (l > RW_LONG) rw_warp_copy(text + d, w.seq_pool + w.seq_off[rr * 5 + s], l, lane);
+        }
+    }
+}
+
+// The resident compare result as the debug writers read it; names uploaded into rb[W_NAMES], ids as in avk_compare_records_bgzf
+static int region_view_device(avk_ctx *ctx, const char *who, const char *const *contig_names, uint32_t n_contigs, const uint64_t *region_id,
+                              const uint64_t *out_len, RegionView &w) {
+    std::string &err = ctx->err;
+    if (!ctx->have_batch || !ctx->have_result) {
+        err = std::string(who) + (ctx->have_merge ? ": the resident result is a merge result, not a compare result" : ": no compare result is resident (run avk_compare_run_resident first)");
+        return AVK_ERR_INVALID;
+    }
+    if ((!contig_names && n_contigs) || !out_len) { err = std::string(who) + ": bad arguments"; return AVK_ERR_INVALID; }
+    if (!region_id && !ctx->ids_resident) { err = std::string(who) + ": the batch was uploaded, so its region ids must be given"; return AVK_ERR_INVALID; }
+    const int rc = upload_names(ctx, who, contig_names, n_contigs, nullptr, 0, true, w.nt);
+    if (rc != AVK_OK) return rc;
+    DevBuf *rb = ctx->rb;
+    const DevBatch db = dev_batch(ctx);
+    w.contig = db.contig; w.start = db.start; w.end = db.end;
+    w.status = (const int *)ctx->status.p;
+    w.rows = (const u64 *)ctx->region_metrics.p;
+    w.seq_off = (const u64 *)ctx->seq_off.p; w.seq_len = (const u32 *)ctx->seq_len.p; w.seq_pool = biased<const u8>(ctx->seq_pool, ctx->seq_base);
+    w.metrics = nullptr; w.n_metrics = 0;
+    if (region_id) {                                              // the caller's ids of the resident bin [lo, lo + n)
+        UPLOAD(rb[W_RID], region_id + ctx->lo, 8 * ctx->n_regions);
+        w.rid = (const u64 *)rb[W_RID].p;
+    } else {
+        w.rid = (const u64 *)ctx->region_id.p;
+    }
+    return AVK_OK;
+}
+// out == NULL: *out_len = the size bound of (header line + `body` bytes); else *text = rb[V_TEXT] with the header line copied in
+// front, for the write pass to fill behind it
+static int debug_finish(avk_ctx *ctx, const char *who, const char *header, u64 body, const uint8_t *out, uint64_t *out_len, u8 **text) {
+    const u64 hl = header ? strlen(header) : 0, len = hl + body;
+    *text = nullptr;
+    if (bgzf_chunks(len) >= 0x7fffffffull) { ctx->err = std::string(who) + ": text too long for one call"; return AVK_ERR_INVALID; }
+    if (!out) { *out_len = bgzf_bound(len); return AVK_OK; }
+    ENSURE(ctx->rb[C_TEXT], len);
+    *text = (u8 *)ctx->rb[C_TEXT].p;
+    if (hl) CK(cudaMemcpyAsync(*text, header, hl, cudaMemcpyHostToDevice, ctx->stream));
+    return AVK_OK;
+}
+
+extern "C" int avk_compare_region_summary_bgzf(avk_ctx *ctx, const char *const *contig_names, uint32_t n_contigs, const uint8_t *metrics, uint32_t n_metrics,
+                                               const uint64_t *region_id, int header, int eof, uint8_t *out, uint64_t cap, uint64_t *out_len) {
+    static const char *who = "avk_compare_region_summary_bgzf";
+    if (!ctx) return AVK_ERR_INVALID;
+    if (!metrics && n_metrics) { ctx->err = std::string(who) + ": bad arguments"; return AVK_ERR_INVALID; }
+    for (uint32_t q = 0; q < n_metrics; ++q)
+        if (metrics[q] > 4) { ctx->err = std::string(who) + ": metric code " + std::to_string(metrics[q]) + " (0 GT .. 4 RECORD_BP)"; return AVK_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->device));
+    RegionView w;
+    int rc = region_view_device(ctx, who, contig_names, n_contigs, region_id, out_len, w);
+    if (rc != AVK_OK) return rc;
+    if (!ctx->result_has_rows) { ctx->err = std::string(who) + ": per-region metric rows were not kept by the last pass (AVK_CMP_KEEP_REGION_ROWS)"; return AVK_ERR_INVALID; }
+    DevBuf *rb = ctx->rb;
+    const u64 n = ctx->n_regions;
+    ENSURE(rb[W_MISC], 64 + n_metrics);
+    unsigned long long *d_misc = (unsigned long long *)rb[W_MISC].p;     // [0] contig out of range, then the metric list
+    if (n_metrics) CK(cudaMemcpyAsync((u8 *)rb[W_MISC].p + 64, metrics, n_metrics, cudaMemcpyHostToDevice, ctx->stream));
+    w.metrics = (const u8 *)rb[W_MISC].p + 64; w.n_metrics = n_metrics;
+    // count pass and the scan of the per-region line counts
+    ENSURE(rb[W_CNT], 8 * (n + 1));
+    u64 *line_off = (u64 *)rb[W_CNT].p;
+    CK(cudaMemsetAsync(d_misc, 0, 8, ctx->stream));
+    size_t need = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, need, line_off, line_off, n + 1, ctx->stream);
+    ENSURE(ctx->scan_tmp, need);
+    k_rs_count<<<(unsigned)((n + 1 + 255) / 256), 256, 0, ctx->stream>>>(w, n, n_contigs, line_off, d_misc);
+    CK(cub::DeviceScan::ExclusiveSum(ctx->scan_tmp.p, need, line_off, line_off, n + 1, ctx->stream));
+    unsigned long long h[2] = {0, 0};
+    CK(cudaMemcpyAsync(&h[0], d_misc, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&h[1], line_off + n, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->launches += 2;
+    CK(cudaGetLastError());
+    if (h[0]) { ctx->err = std::string(who) + ": a region's contig is not below n_contigs"; return AVK_ERR_INVALID; }
+    const u64 n_lines = h[1];
+    // length pass and the scan of the line lengths
+    ENSURE(rb[W_LEN], 8 * (n_lines + 1));
+    ENSURE(rb[W_REG], 4 * n_lines);
+    u64 *off = (u64 *)rb[W_LEN].p;
+    u32 *reg = (u32 *)rb[W_REG].p;
+    need = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, need, off, off, n_lines + 1, ctx->stream);
+    ENSURE(ctx->scan_tmp, need);
+    k_rs_len<<<(unsigned)((n_lines + 1 + 255) / 256), 256, 0, ctx->stream>>>(w, n, n_lines, line_off, reg, off);
+    CK(cub::DeviceScan::ExclusiveSum(ctx->scan_tmp.p, need, off, off, n_lines + 1, ctx->stream));
+    u64 body = 0;
+    CK(cudaMemcpyAsync(&body, off + n_lines, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->launches += 2;
+    CK(cudaGetLastError());
+    const char *hdr = header ? avk_writers::REGION_SUMMARY_HEADER : nullptr;
+    u8 *text = nullptr;
+    rc = debug_finish(ctx, who, hdr, body, out, out_len, &text);
+    if (rc != AVK_OK || !text) return rc;
+    if (n_lines) {
+        k_rs_write<<<(unsigned)((n_lines + 255) / 256), 256, 0, ctx->stream>>>(w, n_lines, reg, line_off, off, hdr ? strlen(hdr) : 0, text);
+        ctx->launches += 1;
+        CK(cudaGetLastError());
+    }
+    return bgzf_compress_device(ctx, (hdr ? strlen(hdr) : 0) + body, eof != 0, out, cap, out_len);
+}
+
+extern "C" int avk_compare_region_sequences_bgzf(avk_ctx *ctx, const char *const *contig_names, uint32_t n_contigs, const uint64_t *region_id,
+                                                 int header, int eof, uint8_t *out, uint64_t cap, uint64_t *out_len) {
+    static const char *who = "avk_compare_region_sequences_bgzf";
+    if (!ctx) return AVK_ERR_INVALID;
+    CK(cudaSetDevice(ctx->device));
+    RegionView w;
+    int rc = region_view_device(ctx, who, contig_names, n_contigs, region_id, out_len, w);
+    if (rc != AVK_OK) return rc;
+    if (!ctx->result_has_seq) {
+        ctx->err = std::string(who) + ": the last pass kept no sequence bundle (AVK_CMP_KEEP_SEQUENCES, or enable_sequences with the seq_* outputs)";
+        return AVK_ERR_INVALID;
+    }
+    DevBuf *rb = ctx->rb;
+    const u64 n = ctx->n_regions;
+    ENSURE(rb[W_MISC], 64);
+    unsigned long long *d_misc = (unsigned long long *)rb[W_MISC].p;     // [0] contig out of range
+    ENSURE(rb[W_LEN], 8 * (n + 1));
+    u64 *off = (u64 *)rb[W_LEN].p;
+    CK(cudaMemsetAsync(d_misc, 0, 8, ctx->stream));
+    size_t need = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, need, off, off, n + 1, ctx->stream);
+    ENSURE(ctx->scan_tmp, need);
+    k_rq_len<<<(unsigned)((n + 1 + 255) / 256), 256, 0, ctx->stream>>>(w, n, n_contigs, off, d_misc);
+    CK(cub::DeviceScan::ExclusiveSum(ctx->scan_tmp.p, need, off, off, n + 1, ctx->stream));
+    unsigned long long h[2] = {0, 0};
+    CK(cudaMemcpyAsync(&h[0], d_misc, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&h[1], off + n, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->launches += 2;
+    CK(cudaGetLastError());
+    if (h[0]) { ctx->err = std::string(who) + ": a region's contig is not below n_contigs"; return AVK_ERR_INVALID; }
+    const u64 body = h[1];
+    const char *hdr = header ? avk_writers::REGION_SEQUENCES_HEADER : nullptr;
+    u8 *text = nullptr;
+    rc = debug_finish(ctx, who, hdr, body, out, out_len, &text);
+    if (rc != AVK_OK || !text) return rc;
+    if (body) {
+        k_rq_write<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(w, n, off, hdr ? strlen(hdr) : 0, text);
+        ctx->launches += 1;
+        CK(cudaGetLastError());
+    }
+    return bgzf_compress_device(ctx, (hdr ? strlen(hdr) : 0) + body, eof != 0, out, cap, out_len);
 }
 
 // ---- outputs of the resident merge, formatted on the device (avk_writers.h::merge_records_text / merge_regions_text and the
@@ -3917,33 +4285,15 @@ static int merge_view_device(avk_ctx *ctx, const char *who, const char *const *c
     if (!contig_names && n_contigs) { err = std::string(who) + ": bad arguments"; return AVK_ERR_INVALID; }
     if (need_ids && !region_id && !ctx->ids_resident) { err = std::string(who) + ": the batch was uploaded, so its region ids must be given"; return AVK_ERR_INVALID; }
     const u64 n = ctx->n_regions, K = ctx->n_inputs;
-    std::vector<u64> tab(n_contigs + 1 + (labels ? K + 1 : 0), 0);
-    std::string packed;
-    for (u32 c = 0; c < n_contigs; ++c) {
-        if (!contig_names[c]) { err = std::string(who) + ": null contig name"; return AVK_ERR_INVALID; }
-        packed += contig_names[c];
-        tab[c + 1] = packed.size();
-    }
-    const u64 names_len = packed.size();
-    if (labels) {
-        u64 *lt = tab.data() + n_contigs + 1;
-        for (u64 k = 0; k < K; ++k) {
-            if (!labels[k]) { err = std::string(who) + ": null input label"; return AVK_ERR_INVALID; }
-            packed += labels[k];
-            lt[k + 1] = packed.size() - names_len;
-        }
-    }
+    NameTable nt;
+    const int rc = upload_names(ctx, who, contig_names, n_contigs, labels, K, false, nt);
+    if (rc != AVK_OK) return rc;
     DevBuf *rb = ctx->rb;
-    const size_t tab_bytes = 8 * tab.size();
-    ENSURE(rb[W_NAMES], tab_bytes + packed.size());
-    CK(cudaMemcpyAsync(rb[W_NAMES].p, tab.data(), tab_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    if (!packed.empty()) CK(cudaMemcpyAsync((u8 *)rb[W_NAMES].p + tab_bytes, packed.data(), packed.size(), cudaMemcpyHostToDevice, ctx->stream));
     const DevBatch db = dev_batch(ctx);
     w.var_off = db.var_off; w.contig = db.contig; w.start = db.start; w.end = db.end; w.pos = db.pos; w.aoff = db.aoff; w.l0 = db.l0; w.l1 = db.l1;
     w.zyg = db.zyg; w.vtype = db.vtype; w.pool = db.pool;
     w.status = (const int *)ctx->status.p; w.cls = (const u8 *)ctx->m_cls.p; w.n_idx = (const u8 *)ctx->m_nidx.p; w.idx = (const u8 *)ctx->m_idx.p;
-    w.name_off = (const u64 *)rb[W_NAMES].p; w.label_off = w.name_off + n_contigs + 1;
-    w.names = (const char *)rb[W_NAMES].p + tab_bytes; w.labels = w.names + names_len;
+    w.name_off = nt.name_off; w.label_off = nt.label_off; w.names = nt.names; w.labels = nt.labels;
     w.K = (u32)K;
     w.rid = nullptr;
     if (need_ids) {

@@ -8,7 +8,9 @@
 //     avk_merge_records_write (VariantMerger::write_variants, src/writers/variant_merger.rs:198-287: body lines of
 //     passing.vcf.gz), avk_merge_regions_write (write_region :294-309: regions.bed / failed_regions.bed) and
 //     avk_merge_summary_write (MergeSummaryWriter, src/writers/merge_summary.rs:56-112), whose ordering and formatting
-//     avk_merge_summary_rows_write shares for the per-key counts the device computes (avk_merge_summary_counts).
+//     avk_merge_summary_rows_write shares for the per-key counts the device computes (avk_merge_summary_counts);
+//   * the debug folder of `aardvark compare` (avk_region_summary_write / avk_region_sequences_write): region_summary.tsv.gz
+//     and region_sequences.tsv.gz, one block per solved region, in this library's layout (see REGION_SUMMARY_HEADER).
 // Plain C++17, no CUDA: the counters and labels were computed on the device, these functions only format them.
 #pragma once
 #include <charconv>
@@ -156,6 +158,61 @@ static inline std::string vcf_records_text(const avk_region_batch *b, uint32_t s
             o += std::to_string((int32_t)b->region_id[r]);                                           // `region_id as i32` (:214)
             o += '\n';
         }
+    return o;
+}
+
+// ---- the debug folder of `aardvark compare`: region_summary.tsv.gz and region_sequences.tsv.gz -------------------------
+// This library's layout (SURVEY Appendix C, summary.tsv's conventions), not pinned by a reference fixture: the two header
+// lines are kept here, in one place, so that they can be checked against src/writers/region_summary.rs:119-138 and
+// region_sequence.rs:18-46 in one edit.  One block per solved region (status 0) in batch order; region_id as the full u64;
+// coordinates chrom:start+1-end (coordinates.rs:73-78); tab-separated, each line ended by '\n'.
+static const char REGION_SUMMARY_HEADER[] = "region_id\tcoordinates\tcomparison\ttruth_tp\ttruth_fn\tquery_tp\tquery_fp\ttruth_fn_gt\tquery_fp_gt\n";
+static const char REGION_SEQUENCES_HEADER[] = "region_id\tcoordinates\tref_seq\ttruth_seq1\ttruth_seq2\tquery_seq1\tquery_seq2\n";
+
+// a contig name both debug writers can print without quoting: no tab, '"', CR or LF
+static inline bool plain_name(const char *s) {
+    for (const char *c = s; *c; ++c) if (*c == '\t' || *c == '"' || *c == '\r' || *c == '\n') return false;
+    return true;
+}
+static inline void region_key(std::string &o, const avk_region_batch *b, const char *const *contig_names, uint64_t r) {
+    o += std::to_string(b->region_id[r]); o += '\t';
+    o += contig_names[b->contig[r]]; o += ':'; o += std::to_string((uint64_t)b->start[r] + 1); o += '-'; o += std::to_string(b->end[r]);
+}
+// per solved region of [lo, hi), per requested metric: the joint group's {tp, fn, qtp, qfp} at METRIC_COL and, on GT lines,
+// truth_fn_gt / query_fp_gt (empty fields otherwise).  No recall / precision / F1.
+static inline std::string region_summary_text(const avk_region_batch *b, const int32_t *status, const uint64_t *region_metrics,
+                                              const char *const *contig_names, const uint8_t *metrics, uint32_t n_metrics, bool header,
+                                              uint64_t lo, uint64_t hi) {
+    std::string o;
+    if (header) o += REGION_SUMMARY_HEADER;
+    for (uint64_t r = lo; r < hi; ++r) {
+        if (status[r] != 0) continue;
+        const uint64_t *row = region_metrics + r * (uint64_t)(AVK_N_GROUPS * AVK_N_METRICS);
+        for (uint32_t q = 0; q < n_metrics; ++q) {
+            const int m = metrics[q];
+            const Row4 c = row_of(row, 0, m);
+            region_key(o, b, contig_names, r);
+            o += '\t'; o += METRIC_NAMES[m];
+            for (uint64_t x : {c.tp, c.fn, c.qtp, c.qfp}) { o += '\t'; o += std::to_string(x); }
+            o += '\t'; if (m == 0) o += std::to_string(c.fn_gt);
+            o += '\t'; if (m == 0) o += std::to_string(c.fp_gt);
+            o += '\n';
+        }
+    }
+    return o;
+}
+// per solved region of [lo, hi): the five SequenceBundle strings (ref, truth1, truth2, query1, query2), string s of region r
+// at seq_pool[seq_off[r*5+s] ..+ seq_len[r*5+s]], as raw bytes
+static inline std::string region_sequences_text(const avk_region_batch *b, const int32_t *status, const uint64_t *seq_off, const uint32_t *seq_len,
+                                                const uint8_t *seq_pool, const char *const *contig_names, bool header, uint64_t lo, uint64_t hi) {
+    std::string o;
+    if (header) o += REGION_SEQUENCES_HEADER;
+    for (uint64_t r = lo; r < hi; ++r) {
+        if (status[r] != 0) continue;
+        region_key(o, b, contig_names, r);
+        for (int s = 0; s < 5; ++s) { o += '\t'; o.append((const char *)seq_pool + seq_off[r * 5 + s], seq_len[r * 5 + s]); }
+        o += '\n';
+    }
     return o;
 }
 

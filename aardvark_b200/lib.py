@@ -116,6 +116,7 @@ EXPORTED_SYMBOLS = [
     "avk_compare_records_bgzf",
     "avk_merge_upload_range", "avk_merge_run_resident", "avk_merge_download", "avk_merge_records_bgzf", "avk_merge_regions_bgzf",
     "avk_merge_summary_counts", "avk_merge_summary_rows_write",
+    "avk_region_summary_write", "avk_region_sequences_write", "avk_compare_region_summary_bgzf", "avk_compare_region_sequences_bgzf",
 ]
 
 
@@ -280,10 +281,12 @@ class Solver:
         else:
             self._check(self._lib.avk_compare_upload_range(self._ctx, C.byref(cb), lo, hi), "avk_compare_upload_range")
 
-    def run_resident(self, cfg: CompareConfig = None, region_metrics: bool = False):
+    def run_resident(self, cfg: CompareConfig = None, region_metrics: bool = False, sequences: bool = False):
         """One pass over the resident batch.  region_metrics=True keeps the per-region metric rows on the device so
-        that download() can return them."""
-        cc = compare_cfg(cfg or CompareConfig(enable_sequences=False), abi.CMP_KEEP_REGION_ROWS if region_metrics else 0)
+        that download() and writers.region_summary_bgzf can use them; sequences=True (needs cfg.enable_sequences) fills the
+        sequence bundle on the device for writers.region_sequences_bgzf (AVK_CMP_KEEP_SEQUENCES; a slower pass)."""
+        flags = (abi.CMP_KEEP_REGION_ROWS if region_metrics else 0) | (abi.CMP_KEEP_SEQUENCES if sequences else 0)
+        cc = compare_cfg(cfg or CompareConfig(enable_sequences=False), flags)
         self._check(self._lib.avk_compare_run_resident(self._ctx, C.byref(cc)), "avk_compare_run_resident")
 
     def result_device_view(self) -> abi.CompareDevView:

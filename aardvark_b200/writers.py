@@ -27,6 +27,10 @@ def _bind():
     lib.avk_merge_regions_write.argtypes = [C.POINTER(abi.RegionBatch), C.POINTER(abi.MergeOut), names, C.c_uint32, C.c_int, C.c_uint64, C.c_uint64] + t
     lib.avk_merge_summary_write.argtypes = [C.POINTER(abi.RegionBatch), C.POINTER(abi.MergeOut), names, C.c_int, C.c_int] + t
     lib.avk_merge_summary_rows_write.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, names, C.c_int, C.c_int] + t
+    lib.avk_region_summary_write.argtypes = [C.POINTER(abi.RegionBatch), C.c_void_p, C.c_void_p, names, C.c_uint32, C.c_void_p, C.c_uint32, C.c_int,
+                                             C.c_uint64, C.c_uint64] + t
+    lib.avk_region_sequences_write.argtypes = [C.POINTER(abi.RegionBatch), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, names, C.c_uint32, C.c_int,
+                                               C.c_uint64, C.c_uint64] + t
     return lib
 
 
@@ -216,3 +220,72 @@ def merge_summary_text(rows, n_inputs, labels, csv=False, header=True) -> str:
     lab = _c_names(labels)
     return _text(lambda buf, cap, n: lib.avk_merge_summary_rows_write(rows.ctypes.data if rows.size else None, rows.size, n_inputs, lab,
                                                                       1 if csv else 0, 1 if header else 0, buf, cap, n))
+
+
+# ---- the debug folder of `aardvark compare`: region_summary.tsv.gz and region_sequences.tsv.gz ----------------------------
+def _metric_codes(metrics):
+    return np.asarray([METRICS[m] if isinstance(m, str) else int(m) for m in metrics] or [0], dtype=np.uint8), len(metrics)
+
+
+def region_summary_lines(batch, contig_names, outputs, metrics=tuple(METRICS), header=True, lo=0, hi=None) -> str:
+    """avk_region_summary_write: region_summary.tsv of regions [lo, hi) -- per solved region one line per metric (names or codes
+    0 GT .. 4 RECORD_BP) with the joint group's counters of outputs.region_metrics."""
+    lib = _bind()
+    hi = batch.n_regions if hi is None else hi
+    cb = batch.to_c()
+    names = _c_names(contig_names)
+    codes, nm = _metric_codes(metrics)
+    return _text(lambda buf, cap, n: lib.avk_region_summary_write(C.byref(cb), outputs.status.ctypes.data, outputs.region_metrics.ctypes.data, names,
+                                                                  len(contig_names), codes.ctypes.data, nm, 1 if header else 0, lo, hi, buf, cap, n))
+
+
+def region_sequence_lines(batch, contig_names, outputs, header=True, lo=0, hi=None) -> bytes:
+    """avk_region_sequences_write: region_sequences.tsv of regions [lo, hi) -- per solved region the five strings of the
+    sequence bundle in outputs (CompareOutputs with seq_off).  Raw bytes: the sequences are written as they are."""
+    lib = _bind()
+    hi = batch.n_regions if hi is None else hi
+    cb = batch.to_c()
+    names = _c_names(contig_names)
+    call = lambda buf, cap, n: lib.avk_region_sequences_write(C.byref(cb), outputs.status.ctypes.data, outputs.seq_off.ctypes.data, outputs.seq_len.ctypes.data,
+                                                              outputs.seq_pool.ctypes.data, names, len(contig_names), 1 if header else 0, lo, hi, buf, cap, n)
+    n = C.c_uint64(0)
+    if call(None, 0, C.byref(n)) != 0:
+        raise AvkError("avk_region_sequences_write failed")
+    buf = C.create_string_buffer(int(n.value) + 1)
+    if call(buf, int(n.value), C.byref(n)) != 0:
+        raise AvkError("avk_region_sequences_write failed")
+    return buf.raw[:int(n.value)]
+
+
+def _debug_bgzf_fns(lib):
+    t = [C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+    names = C.POINTER(C.c_char_p)
+    lib.avk_compare_region_summary_bgzf.argtypes = [C.c_void_p, names, C.c_uint32, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint64), C.c_int, C.c_int] + t
+    lib.avk_compare_region_sequences_bgzf.argtypes = [C.c_void_p, names, C.c_uint32, C.POINTER(C.c_uint64), C.c_int, C.c_int] + t
+    return lib.avk_compare_region_summary_bgzf, lib.avk_compare_region_sequences_bgzf
+
+
+def region_summary_bgzf(solver, contig_names, metrics=tuple(METRICS), region_ids=None, header=True, eof=True) -> bytes:
+    """avk_compare_region_summary_bgzf: region_summary.tsv.gz of the solver's resident compare result (rows kept:
+    run_resident(region_metrics=True) or compare_batch with region_metrics), formatted and compressed on the device -- the same
+    bytes as bgzf_compress(solver, region_summary_lines(...)) over the resident bin.  region_ids, eof: as in vcf_records_bgzf;
+    header=True on the first bin only."""
+    fn = _debug_bgzf_fns(solver._lib)[0]
+    names = _c_names(contig_names)
+    codes, nm = _metric_codes(metrics)
+    rid = None if region_ids is None else np.ascontiguousarray(region_ids, dtype=np.uint64)
+    rid_p = abi.ptr(rid)
+    return _bgzf_call(solver, "avk_compare_region_summary_bgzf", lambda buf, cap, n: fn(solver._ctx, names, len(contig_names), codes.ctypes.data, nm, rid_p,
+                                                                                         1 if header else 0, 1 if eof else 0, buf, cap, n))
+
+
+def region_sequences_bgzf(solver, contig_names, region_ids=None, header=True, eof=True) -> bytes:
+    """avk_compare_region_sequences_bgzf: region_sequences.tsv.gz of the solver's resident compare result (bundle kept:
+    run_resident(cfg with enable_sequences, sequences=True) or compare_batch with the bundle), formatted and compressed on the
+    device -- the same bytes as bgzf_compress(solver, region_sequence_lines(...)) over the resident bin."""
+    fn = _debug_bgzf_fns(solver._lib)[1]
+    names = _c_names(contig_names)
+    rid = None if region_ids is None else np.ascontiguousarray(region_ids, dtype=np.uint64)
+    rid_p = abi.ptr(rid)
+    return _bgzf_call(solver, "avk_compare_region_sequences_bgzf", lambda buf, cap, n: fn(solver._ctx, names, len(contig_names), rid_p, 1 if header else 0,
+                                                                                           1 if eof else 0, buf, cap, n))

@@ -175,6 +175,13 @@ typedef struct avk_compare_cfg {
 /* avk_compare_run_resident: keep the per-region GroupTypeMetrics rows (2288 B per region) on the device so that
  * avk_compare_download can return out->region_metrics.  avk_compare_batch* decide from out->region_metrics != NULL. */
 #define AVK_CMP_KEEP_REGION_ROWS 1u
+/* avk_compare_run_resident: fill the sequence bundle (compare_benchmark.rs:159-185) of the resident bin on the device, in the
+ * layout avk_compare_seq_offsets gives the bin (offsets from 0), so that avk_compare_region_sequences_bgzf can write it.
+ * Needs enable_sequences != 0 (the flag without it is refused).  Without the flag the pass is exactly the plain one: the
+ * bundle makes the team stage emit the strings, so every cluster the closed forms and the thread stage would finish goes
+ * there instead: measured on a B200, the chr20-shaped pass (115 k clusters) takes 6.9 ms with the bundle against 3.3 ms with
+ * the rows only.  avk_compare_batch* decide from the out->seq_* pointers. */
+#define AVK_CMP_KEEP_SEQUENCES 2u
 
 /* MergeConfig, src/merge_solver.rs:62-84 */
 typedef struct avk_merge_cfg {
@@ -425,6 +432,41 @@ int avk_vcf_records_write(const avk_region_batch *batch, uint32_t side, const ch
 int avk_compare_records_bgzf(avk_ctx *ctx, uint32_t side, const char *const *contig_names, uint32_t n_contigs,
                              const uint64_t *region_id, const uint8_t *header, uint64_t header_len, int eof,
                              uint8_t *out, uint64_t cap, uint64_t *out_len);
+
+/* ---- the debug folder of `aardvark compare` (SURVEY Appendix C): region_summary.tsv.gz (src/writers/region_summary.rs) and
+ * region_sequences.tsv.gz (region_sequence.rs).  The column layout is this library's (the header lines are in
+ * csrc/avk_writers.h) and is not pinned by a reference fixture.  Tab-separated lines ended by '\n'; header != 0 puts one
+ * header line first.  One block per SOLVED region (status == 0) of [lo, hi) in batch order (an unsolved region has no
+ * benchmark, src/main.rs:259-262); region_id as the full u64 in decimal; coordinates chrom:start+1-end (coordinates.rs:73-78,
+ * e.g. start 100, end 250 on chr1 -> chr1:101-250).  A contig name containing a tab, '"', CR or LF, a null name, or a region
+ * whose contig is >= n_contigs fails the call (AVK_ERR_INVALID).  Host only; buf == NULL: *len receives the size needed.
+ * avk_region_summary_write: per solved region, one line per metric listed (0 GT, 1 HAP, 2 WEIGHTED_HAP, 3 BASEPAIR,
+ *   4 RECORD_BP, in the order given; a code above 4 fails the call): region_id, coordinates, the metric's name, truth_tp,
+ *   truth_fn, query_tp, query_fp of the region's joint group (group 0 of region_metrics[r]), then truth_fn_gt / query_fp_gt
+ *   on GT lines and two empty fields on the others.  No recall / precision / F1 columns.
+ * avk_region_sequences_write: per solved region one line: region_id, coordinates and the five bundle strings ref, truth1,
+ *   truth2, query1, query2 (string s of region r = seq_pool[seq_off[r*5+s] ..+ seq_len[r*5+s]]) as raw bytes. */
+int avk_region_summary_write(const avk_region_batch *batch, const int32_t *status, const uint64_t *region_metrics,
+                             const char *const *contig_names, uint32_t n_contigs, const uint8_t *metrics, uint32_t n_metrics, int header,
+                             uint64_t lo, uint64_t hi, char *buf, uint64_t cap, uint64_t *len);
+int avk_region_sequences_write(const avk_region_batch *batch, const int32_t *status, const uint64_t *seq_off, const uint32_t *seq_len,
+                               const uint8_t *seq_pool, const char *const *contig_names, uint32_t n_contigs, int header,
+                               uint64_t lo, uint64_t hi, char *buf, uint64_t cap, uint64_t *len);
+/* The same two files of the resident compare result, formatted and BGZF-compressed on the device: out = byte for byte
+ * avk_bgzf_compress(avk_region_summary_write(batch, status, region_metrics, contig_names, n_contigs, metrics, n_metrics,
+ * header, lo, lo + n)), resp. avk_bgzf_compress(avk_region_sequences_write(batch, status, seq_off, seq_len, seq_pool,
+ * contig_names, n_contigs, header, lo, lo + n)), for the resident bin [lo, lo + n) -- pass header != 0 for the first bin only.
+ * region_id, eof, out == NULL (an upper bound of the size) and cap < size (AVK_ERR_OOM with *out_len = the exact size) behave
+ * as in avk_compare_records_bgzf.
+ * The summary needs the per-region rows on the device: a resident run with AVK_CMP_KEEP_REGION_ROWS, or avk_compare_batch /
+ * avk_compare_batch_range called with out->region_metrics.  The sequences need the bundle on the device: a resident run with
+ * AVK_CMP_KEEP_SEQUENCES, or avk_compare_batch* called with enable_sequences and the out->seq_* outputs.  Both fail with
+ * AVK_ERR_INVALID (and a message; the context stays usable) when no compare result is resident (none yet, or a merge
+ * result), when the rows resp. the bundle were not kept by the last pass, and on the argument errors of the host writers. */
+int avk_compare_region_summary_bgzf(avk_ctx *ctx, const char *const *contig_names, uint32_t n_contigs, const uint8_t *metrics, uint32_t n_metrics,
+                                    const uint64_t *region_id, int header, int eof, uint8_t *out, uint64_t cap, uint64_t *out_len);
+int avk_compare_region_sequences_bgzf(avk_ctx *ctx, const char *const *contig_names, uint32_t n_contigs, const uint64_t *region_id,
+                                      int header, int eof, uint8_t *out, uint64_t cap, uint64_t *out_len);
 
 /* The outputs of `aardvark merge` that are functions of avk_merge_out (host only; regions with status != 0 are skipped as
  * src/main.rs:507-524 skips failed regions; `result->status` may be NULL = all solved):
