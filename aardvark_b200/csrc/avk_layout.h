@@ -30,6 +30,10 @@ enum { AL_UNSET = 0, AL_REF = 1, AL_ALT = 2 };
 // a CTA adds to slot blockIdx.x % TOT_SLOTS (u64 atomics in L2, little contention), k_fold_slots sums the slots.
 enum { TOT_SLOTS = 128, TOT_COLS = AVK_N_GROUPS * AVK_N_METRICS, TOT_MASK = TOT_COLS, TOT_SOLVED = TOT_COLS + 1,
        TOT_ERRORS = TOT_COLS + 2, TOT_STRIDE = TOT_COLS + 6 };
+// Per-stratum sums, added at the same places as the totals: STRAT_SLOTS partial tables [n_strata][TOT_COLS] (fewer than
+// TOT_SLOTS so that 1,000 strata of the list path stay at 36 MB); a CTA adds to slot blockIdx.x % STRAT_SLOTS, k_fold_strata
+// sums the slots.
+enum { STRAT_SLOTS = 16 };
 
 static AVK_HD inline bool type_supported(int t) {   // SUPPORTED_VARIANT_TYPES waffle_solver.rs:82-91
     return t == AVK_VT_SNV || t == AVK_VT_INSERTION || t == AVK_VT_DELETION || t == AVK_VT_INDEL ||

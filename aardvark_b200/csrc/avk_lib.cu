@@ -5,7 +5,7 @@
 //   k_compare      one warp per cluster, persistent warps     waffle_solver.rs:122-284
 //   k_merge        one warp per cluster                       merge_solver.rs:110-200
 //   k_wfa_ed       one warp per alignment                     util/sequence_alignment.rs:9-13
-//   k_reduce       sum of per-region metrics                  writers/summary.rs:146-158
+//   k_fold_slots   summary counters, k_fold_strata per stratum  writers/summary.rs:146-158
 //
 // There is NO CPU fallback in this library: every entry point either runs the CUDA path or
 // returns an error code.
@@ -369,6 +369,55 @@ __device__ __forceinline__ void zero_region_outputs(const DevBatch &b, const Dev
     __syncwarp();
 }
 
+// the closed forms' metric entries v = {pairs, ALT copies, weighted by truth / query ALT edit distance, 2 X, 2 x truth /
+// query raw allele space} into one [22]-metric row
+__device__ __forceinline__ void add_closed_form_row(unsigned long long *g, const unsigned long long v[7]) {
+    atomicAdd(g + AVK_M_GT, v[0]); atomicAdd(g + AVK_M_GT + 2, v[0]);
+    atomicAdd(g + AVK_M_HAP, v[1]); atomicAdd(g + AVK_M_HAP + 2, v[1]);
+    atomicAdd(g + AVK_M_WEIGHTED_HAP, v[2]); atomicAdd(g + AVK_M_WEIGHTED_HAP + 2, v[3]);
+    atomicAdd(g + AVK_M_BASEPAIR, v[4]); atomicAdd(g + AVK_M_BASEPAIR + 2, v[4]);
+    atomicAdd(g + AVK_M_RECORD_BP, v[5]); atomicAdd(g + AVK_M_RECORD_BP + 2, v[6]);
+}
+// per-stratum sums of the closed-form clusters of one warp (all 32 lanes call it).  Device lookup: one warp reduction per
+// (variant type, containment mask) present, the (stratum, row) pairs of the mask spread over the lanes.  Caller's list: each
+// cluster adds its own rows to its strata.
+__device__ __forceinline__ void closed_form_strata(const DevStrata &st, u64 r, bool simple, u32 vtype, unsigned long long c0, unsigned long long c1,
+                                                unsigned long long c2, unsigned long long c3, unsigned long long c4, unsigned long long c5,
+                                                unsigned long long c6) {
+    const int lane = lane_id();
+    const unsigned long long cv[7] = {c0, c1, c2, c3, c4, c5, c6};
+    unsigned long long *tab = st.slots + (size_t)(blockIdx.x & (STRAT_SLOTS - 1)) * st.n_strata * TOT_COLS;
+    if (st.st_mask) {
+        const u64 mk = simple ? st.st_mask[r] : 0ull;
+        u32 left = __ballot_sync(AVK_FULL, mk != 0);
+        while (left) {
+            const int src = __ffs(left) - 1;
+            const u32 ty = __shfl_sync(AVK_FULL, vtype, src);
+            const u64 m = __shfl_sync(AVK_FULL, (unsigned long long)mk, src);
+            const bool in = mk == m && vtype == ty;
+            left &= ~__ballot_sync(AVK_FULL, in);
+            unsigned long long v[7];
+#pragma unroll
+            for (int k = 0; k < 7; ++k) {
+                v[k] = in ? cv[k] : 0ull;
+#pragma unroll
+                for (int o = 16; o; o >>= 1) v[k] += __shfl_xor_sync(AVK_FULL, v[k], o);
+            }
+            for (int job = lane; job < 2 * __popcll(m); job += 32) {
+                u64 mm = m;
+                for (int k = job >> 1; k; --k) mm &= mm - 1;
+                add_closed_form_row(tab + (size_t)(__ffsll((long long)mm) - 1) * TOT_COLS + ((job & 1) ? (1 + ty) * AVK_N_METRICS : 0), v);
+            }
+        }
+    } else if (simple) {
+        for (u64 s = st.strat_off[r], e = st.strat_off[r + 1]; s < e; ++s) {
+            unsigned long long *g = tab + (size_t)st.strat_idx[s] * TOT_COLS;
+            add_closed_form_row(g, cv);
+            add_closed_form_row(g + (1 + vtype) * AVK_N_METRICS, cv);
+        }
+    }
+}
+
 // ---- closed form for the commonest cluster shape ------------------------------------------------------------
 // One truth and one query record that are the same variant -- same position, reference span, ALT bytes, (supported) type
 // label and number of ALT copies -- where the variant is a substitution that changes the base, or an anchored pure
@@ -387,6 +436,8 @@ __device__ __forceinline__ void zero_region_outputs(const DevBatch &b, const Dev
 // sequence bundle requested -- goes to the search kernels through `work_list`.
 // Clusters with at least `dense_n` variants skip the search / score pair: they go to list `dense`, which the fused
 // stage starts on first (the longest searches of a batch are among them).
+// STRATA: the pass sums strata too (a separate instantiation, so that a plain pass runs exactly the code without them)
+template <bool STRATA>
 __global__ void __launch_bounds__(256) k_compare_simple(DevBatch b, DevCompareOut out, avk_compare_cfg cfg, u64 n, u32 *work_list,
                                                         u32 *work_ctr, u32 *dense, u32 *dense_ctr, int dense_n, u64 *work_key) {
     const int lane = lane_id();
@@ -510,17 +561,14 @@ __global__ void __launch_bounds__(256) k_compare_simple(DevBatch b, DevCompareOu
                     for (int o = 16; o; o >>= 1) v[k] += __shfl_xor_sync(AVK_FULL, v[k], o);
                 }
                 if (lane < 2) {                                          // lane 0: joint row, lane 1: the type's row
-                    unsigned long long *g = slot + (lane == 0 ? 0 : (1 + ty) * AVK_N_METRICS);
-                    atomicAdd(g + AVK_M_GT, v[0]); atomicAdd(g + AVK_M_GT + 2, v[0]);
-                    atomicAdd(g + AVK_M_HAP, v[1]); atomicAdd(g + AVK_M_HAP + 2, v[1]);
-                    atomicAdd(g + AVK_M_WEIGHTED_HAP, v[2]); atomicAdd(g + AVK_M_WEIGHTED_HAP + 2, v[3]);
-                    atomicAdd(g + AVK_M_BASEPAIR, v[4]); atomicAdd(g + AVK_M_BASEPAIR + 2, v[4]);
-                    atomicAdd(g + AVK_M_RECORD_BP, v[5]); atomicAdd(g + AVK_M_RECORD_BP + 2, v[6]);
+                    add_closed_form_row(slot + (lane == 0 ? 0 : (1 + ty) * AVK_N_METRICS), v);
                     if (lane == 0) { atomicAdd(slot + TOT_SOLVED, (unsigned long long)__popc(same)); atomicOr(slot + TOT_MASK, (unsigned long long)supported); }
                 }
             }
         }
-        // metric rows [13][22] (only when the caller wants per-region rows or strata), written by the whole warp per
+        if (STRATA)
+            closed_form_strata(*out.strata, r, simple, vtype, (unsigned long long)npairs, s_c, s_wT, s_wQ, 2ull * s_X, 2ull * s_rT, 2ull * s_rQ);
+        // metric rows [13][22] (only when the caller wants per-region rows), written by the whole warp per
         // cluster: joint row == the (single) type's row, the rest zero
         u32 todo = out.region_metrics ? __ballot_sync(AVK_FULL, simple) : 0u;
         while (todo) {
@@ -822,11 +870,13 @@ __global__ void __launch_bounds__(128 * TEAMS_PER_CTA, 1) k_compare_team(DevBatc
 // gets SPB_NONE in its slot and is solved from scratch by the team stage.
 enum { SPEC_WARPS = 8 };
 __device__ unsigned long long *g_spec_prof = nullptr;   // AVK_SPEC_PROFILE: per cluster {region, N, pops, load, search, score, metrics + commit} cycles
+template <bool STRATA>
 struct SpecSink {
     const avk_sp::View &V;
     const DevCompareOut &out;
     u64 *row;
     unsigned long long *slot;
+    u32 r;
     __device__ __forceinline__ void variant(int oi, int e, int o) {
         const u32 *rec = (const u32 *)(V.recs + (size_t)VI_SIZE * oi);
         const u32 gv = rec[VI_GV / 4];
@@ -837,13 +887,15 @@ struct SpecSink {
     __device__ __forceinline__ void metric(int g, int m, u64 v) {
         if (row) row[g * AVK_N_METRICS + m] = v;
         if (slot) atomicAdd(slot + g * AVK_N_METRICS + m, (unsigned long long)v);
+        if (STRATA) out.strata->add(r, g * AVK_N_METRICS + m, (unsigned long long)v);
     }
 };
 // lane 0: outputs of a cluster the speculative path has solved completely (as the commit block of k_compare_thread)
+template <bool STRATA>
 __device__ __noinline__ void spec_commit(const avk_sp::View &V, const avk_sp::Shared &S, const DevBatch &b, const DevCompareOut &out, u32 r, unsigned long long *slot) {
     u64 *row = out.region_metrics ? out.region_metrics + (u64)r * (AVK_N_GROUPS * AVK_N_METRICS) : nullptr;
     if (row) for (int i = 0; i < AVK_N_GROUPS * AVK_N_METRICS; ++i) row[i] = 0;
-    SpecSink sink{V, out, row, slot};
+    SpecSink<STRATA> sink{V, out, row, slot, r};
     u32 e1 = 0, e2 = 0;
     uint16_t tm = 0;
     const int rc = avk_sp::commit_metrics(V, S, sink, &e1, &e2, &tm);
@@ -859,6 +911,9 @@ __device__ __noinline__ void spec_commit(const avk_sp::View &V, const avk_sp::Sh
     }
     out.status[r] = rc;
 }
+// STRATA (here and in k_compare_thread): the pass sums strata too -- a separate instantiation, so that a plain pass runs the
+// kernel without the stratum adds of its commit (measured on a B200 at 1000 W: the branch to them alone made both kernels of a plain WGS pass 2-3 % slower)
+template <bool STRATA>
 __global__ void __launch_bounds__(32 * SPEC_WARPS, 1) k_search_spec(DevBatch b, DevCompareOut out, avk_compare_cfg cfg, TierArgs t) {
     using namespace avk_sp;
     const int lane = lane_id(), warp = threadIdx.x >> 5;
@@ -904,7 +959,7 @@ __global__ void __launch_bounds__(32 * SPEC_WARPS, 1) k_search_spec(DevBatch b, 
                 if (scored) {
                     xpops += S.xpops;
                     if (finish_here && metrics_warp(S, X, V, ctr)) {    // metrics + every output right here: nothing is left for the team stage
-                        if (lane == 0) spec_commit(V, S, b, out, r, slot);
+                        if (lane == 0) spec_commit<STRATA>(V, S, b, out, r, slot);
                         nres = SPB_DONE;
                     } else if (lane == 0) {
                         store_result(blob, 0, S.res[S.best_r], n);
@@ -950,11 +1005,13 @@ __global__ void __launch_bounds__(32 * SPEC_WARPS, 1) k_search_spec(DevBatch b, 
 // atomic per warp and round).  A cluster that does not fit the fixed workspace is appended to the reject list -- nothing
 // has been written for it -- and goes through the warp kernels (search / score / fused stages) as before.
 enum { THREAD_TPB = 256, TS_BATCH_MIN = 16 };   // (default of TierArgs::batch_min; swept 1..24 on B200: 14-16 is the flat optimum at every batch size)
+template <bool STRATA>
 struct ThreadSink {
     const avk_ts::Cluster &cl;
     const DevCompareOut &out;
     u64 *row;
     unsigned long long *slot;
+    u32 r;
     __device__ __forceinline__ void variant(int oi, int e, int o) {
         const u32 gv = avk_ts::rec32(cl, oi, VI_GV);
         const bool tr = (avk_ts::rec32(cl, oi, VI_FLAGS) & 0x10000u) != 0;
@@ -964,8 +1021,10 @@ struct ThreadSink {
     __device__ __forceinline__ void metric(int g, int m, u64 v) {
         if (row) row[g * AVK_N_METRICS + m] = v;
         if (slot) atomicAdd(slot + g * AVK_N_METRICS + m, (unsigned long long)v);
+        if (STRATA) out.strata->add(r, g * AVK_N_METRICS + m, (unsigned long long)v);
     }
 };
+template <bool STRATA>
 __global__ void __launch_bounds__(THREAD_TPB, 1) k_compare_thread(DevBatch b, DevCompareOut out, avk_compare_cfg cfg, TierArgs t) {
     using namespace avk_ts;
     const int lane = lane_id();
@@ -998,7 +1057,7 @@ __global__ void __launch_bounds__(THREAD_TPB, 1) k_compare_thread(DevBatch b, De
                     u64 *row = out.region_metrics ? out.region_metrics + (u64)r * (AVK_N_GROUPS * AVK_N_METRICS) : nullptr;
                     if (row) for (int i = 0; i < AVK_N_GROUPS * AVK_N_METRICS; ++i) row[i] = 0;
                     if (rc == AVK_ST_OK) {
-                        ThreadSink sink{S.c, out, row, slot};
+                        ThreadSink<STRATA> sink{S.c, out, row, slot, r};
                         u32 e1 = 0, e2 = 0;
                         uint16_t tm = 0;
                         rc = commit_solution(S, sink, &e1, &e2, &tm);
@@ -1155,45 +1214,15 @@ __global__ void __launch_bounds__(256) k_merge_classify(DevBatch b, DevMergeOut 
     }
 }
 
-// SummaryWriter::add_comparison_benchmark (writers/summary.rs:146-158): thread j sums column j of the
-// [n][286] metric rows (coalesced across the block), one atomicAdd per column per block.
 #define RED_COLS (AVK_N_GROUPS * AVK_N_METRICS)
-__global__ void __launch_bounds__(288) k_reduce(u64 n, const int *status, const u64 *region_metrics, const uint16_t *type_mask,
-                                                unsigned long long *totals, u32 *totals_mask, unsigned long long *solved,
-                                                unsigned long long *errors, const u64 *strat_off, const u32 *strat_idx,
-                                                const u64 *strat_mask, unsigned long long *strat_totals) {
-    const int j = threadIdx.x;
-    unsigned long long acc = 0, ok = 0, bad = 0;
-    u32 mask = 0;
-    // four regions per trip: the status loads, then the row loads, are issued together (the loop is latency-bound otherwise)
-    for (u64 r0 = blockIdx.x; r0 < n; r0 += 4ull * gridDim.x) {
-        bool good[4];
-        unsigned long long v[4];
+// strat_totals[j] = sum over the per-stratum partial tables ([STRAT_SLOTS][cols], cols = n_strata * RED_COLS)
+__global__ void __launch_bounds__(256) k_fold_strata(const unsigned long long *slots, u64 cols, unsigned long long *strat_totals) {
+    for (u64 j = (u64)blockIdx.x * blockDim.x + threadIdx.x; j < cols; j += (u64)gridDim.x * blockDim.x) {
+        unsigned long long acc = 0;
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const u64 r = r0 + (u64)k * gridDim.x;
-            good[k] = r < n && status[r] == AVK_ST_OK;
-        }
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const u64 r = r0 + (u64)k * gridDim.x;
-            v[k] = (good[k] && j < RED_COLS) ? region_metrics[r * RED_COLS + j] : 0ull;
-        }
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const u64 r = r0 + (u64)k * gridDim.x;
-            if (r >= n) break;
-            if (j == 0) { if (good[k]) { ok += 1; mask |= type_mask[r]; } else bad += 1; }
-            acc += v[k];
-            if (strat_off && v[k]) {
-                for (u64 s = strat_off[r]; s < strat_off[r + 1]; ++s) atomicAdd(strat_totals + (u64)strat_idx[s] * RED_COLS + j, v[k]);
-            } else if (strat_mask && v[k]) {
-                for (u64 m = strat_mask[r]; m; m &= m - 1) atomicAdd(strat_totals + (u64)(__ffsll((long long)m) - 1) * RED_COLS + j, v[k]);
-            }
-        }
+        for (int s = 0; s < STRAT_SLOTS; ++s) acc += slots[(size_t)s * cols + j];
+        strat_totals[j] = acc;
     }
-    if (j < RED_COLS && acc) atomicAdd(totals + j, acc);
-    if (j == 0) { atomicAdd(solved, ok); atomicAdd(errors, bad); atomicOr(totals_mask, mask); }
 }
 
 // Stratifications::containments (stratifications.rs:108-118, 197-210) for every region: one thread per region.
@@ -1256,7 +1285,7 @@ struct avk_ctx {
     // batch buffers
     DevBuf region_id, contig, start, end, var_off, pos, vtype, zyg, raw, aoff, l0, l1, pool, alt_ed;
     // outputs
-    DevBuf status, ed1, ed2, region_metrics, type_mask, vexp, vobs, vcls, totals, tot_slots, strat_off, strat_idx, strat_totals,
+    DevBuf status, ed1, ed2, region_metrics, type_mask, vexp, vobs, vcls, totals, tot_slots, strat_off, strat_idx, strat_totals, strat_slots, strat_args,
         seq_off, seq_len, seq_pool, m_cls, m_nidx, m_idx, m_rows, m_perr, m_tasks;
     // workspace
     DevBuf digest, digest_sizes, digest_offs, scan_tmp, blobs, scratch, arena, arena2, counters, fail_a, fail_b, fail_c, fail_d, fail_h, fail_w, fail_x, fail_t, fail_s, shape_key, work_ctr, pair_a_off, pair_b_off, pair_a_len, pair_b_len, pair_ed, pair_pool;
@@ -1273,7 +1302,8 @@ struct avk_ctx {
     bool have_result = false, result_has_rows = false;
     bool result_has_seq = false;    // the last compare pass filled the sequence bundle (seq_off / seq_len / seq_pool, offsets biased by seq_base)
     bool have_merge = false;        // the last pass was a merge: its result (status, m_cls, m_nidx, m_idx) is resident; cleared with have_result
-    bool result_has_contain = false;   // the last pass filled st_mask (a resident run never computes containment)
+    bool result_has_contain = false;   // the last pass filled st_mask (a resident run only with AVK_CMP_STRATA)
+    u32 result_strata = 0;             // the last pass was a resident run with AVK_CMP_STRATA over this many strata (0: it was not)
     u64 lo = 0, n_regions = 0, v_base = 0, n_variants = 0, p_base = 0, pool_bytes = 0;
     u64 seq_base = 0, strat_base = 0;
     u32 n_inputs = 0;
@@ -1384,8 +1414,10 @@ static int configure_kernels(avk_ctx *ctx) {
     SMEM_OPT_IN((k_compare<true, 4, MODE_SCORE>));
     SMEM_OPT_IN((k_compare<true, 1, MODE_FUSED>));
     SMEM_OPT_IN(k_compare_team);
-    SMEM_OPT_IN(k_compare_thread);
-    SMEM_OPT_IN(k_search_spec);
+    SMEM_OPT_IN(k_compare_thread<false>);
+    SMEM_OPT_IN(k_compare_thread<true>);
+    SMEM_OPT_IN(k_search_spec<false>);
+    SMEM_OPT_IN(k_search_spec<true>);
     SMEM_OPT_IN(k_wfa_ed_cta);
     SMEM_OPT_IN((k_merge_pairs<true, 3>));
     SMEM_OPT_IN((k_merge_pairs<true, 1>));
@@ -1482,7 +1514,7 @@ extern "C" void avk_destroy(avk_ctx *ctx) {
     DevBuf *bufs[] = {&ctx->d_contig_ptr, &ctx->d_contig_len, &ctx->region_id, &ctx->contig, &ctx->start, &ctx->end, &ctx->var_off,
                       &ctx->pos, &ctx->vtype, &ctx->zyg, &ctx->raw, &ctx->aoff, &ctx->l0, &ctx->l1, &ctx->pool, &ctx->alt_ed,
                       &ctx->status, &ctx->ed1, &ctx->ed2, &ctx->region_metrics, &ctx->type_mask, &ctx->vexp, &ctx->vobs, &ctx->vcls,
-                      &ctx->totals, &ctx->tot_slots, &ctx->strat_off, &ctx->strat_idx, &ctx->strat_totals, &ctx->seq_off, &ctx->seq_len, &ctx->seq_pool,
+                      &ctx->totals, &ctx->tot_slots, &ctx->strat_off, &ctx->strat_idx, &ctx->strat_totals, &ctx->strat_slots, &ctx->strat_args, &ctx->seq_off, &ctx->seq_len, &ctx->seq_pool,
                       &ctx->m_cls, &ctx->m_nidx, &ctx->m_idx, &ctx->m_rows, &ctx->m_perr, &ctx->m_tasks, &ctx->digest, &ctx->digest_sizes, &ctx->digest_offs, &ctx->scan_tmp, &ctx->blobs, &ctx->scratch, &ctx->arena, &ctx->arena2, &ctx->counters, &ctx->fail_a, &ctx->fail_b, &ctx->fail_c, &ctx->fail_d, &ctx->fail_h, &ctx->fail_w, &ctx->fail_x, &ctx->fail_t, &ctx->fail_s, &ctx->shape_key, &ctx->dense_blobs, &ctx->dense_blobs2, &ctx->spec_prof,
                       &ctx->work_ctr, &ctx->pair_a_off, &ctx->pair_b_off, &ctx->pair_a_len, &ctx->pair_b_len, &ctx->pair_ed, &ctx->pair_pool};
     for (DevBuf *b : bufs) if (b->p) cudaFree(b->p);
@@ -1848,6 +1880,7 @@ static int run_prepare(avk_ctx *ctx, const DevBatch &db) {
     return AVK_OK;
 }
 
+#define DEVICE_LOOKUP_NEEDS "the device containment lookup needs avk_set_stratifications (same number of strata as n_strata, contigs as the reference)"
 // strata sums are requested with a caller-provided membership list (strat_off / strat_idx) or, when strat_off is NULL, through
 // the device containment lookup (avk_set_stratifications)
 static inline bool strata_wanted(const avk_compare_out *out) { return out->strat_totals && out->n_strata; }
@@ -1856,12 +1889,8 @@ struct CompareRun {           // what one compare pass needs to know to launch, 
     DevBatch db;
     DevCompareOut out;
     avk_compare_cfg cfg;
-    bool strata = false;
-    const u64 *strat_off = nullptr;
-    const u32 *strat_idx = nullptr;
-    const u64 *strat_mask = nullptr;   // device containment lookup instead of a caller-provided membership list
     bool want_contain = false;         // compute the containment masks (for the strata sums and / or out->containment)
-    u32 n_strata = 0;
+    DevStrata strata = {};             // host copy of *out.strata
 };
 
 static void launch_stage(avk_ctx *ctx, const CompareRun &R, const Stage &st, const TierArgs &a, int ctas, cudaStream_t strm) {
@@ -1923,7 +1952,8 @@ static int run_compare_pipeline(avk_ctx *ctx, const CompareRun &R) {
         keys = (u64 *)ctx->shape_key.p;
         CK(cudaMemsetAsync(keys, 0xff, 8 * n, ctx->stream));          // unused tail sorts behind every real key
     }
-    k_compare_simple<<<sm * 8, 256, 0, ctx->stream>>>(R.db, R.out, R.cfg, n, LW, ctrs + 12, LX, ctrs + 17, dense_n, keys);
+    if (R.out.strata) k_compare_simple<true><<<sm * 8, 256, 0, ctx->stream>>>(R.db, R.out, R.cfg, n, LW, ctrs + 12, LX, ctrs + 17, dense_n, keys);
+    else k_compare_simple<false><<<sm * 8, 256, 0, ctx->stream>>>(R.db, R.out, R.cfg, n, LW, ctrs + 12, LX, ctrs + 17, dense_n, keys);
     if (keys) {                                                       // W sorted by shape -> fail_s (the first |W| entries are the real ones)
         size_t need = 0;
         cub::DeviceRadixSort::SortPairs(nullptr, need, keys, keys + n, LW, (u32 *)ctx->fail_s.p, (int)n, 0, 64, ctx->stream);
@@ -1944,7 +1974,9 @@ static int run_compare_pipeline(avk_ctx *ctx, const CompareRun &R) {
             ENSURE(blobs, (size_t)dense_cap * avk_sp::SPB_SIZE);
             TierArgs sa = tier_args(ctx, list, in_ctr, spec_ctr, nullptr, 21, 0, nullptr);
             sa.dense_blobs = (u8 *)blobs.p; sa.dense_cap = dense_cap;
-            k_search_spec<<<sm, 32 * SPEC_WARPS, SPEC_WARPS * (sizeof(avk_sp::Shared) + 32 * sizeof(avk_sp::Scratch)), strm>>>(R.db, R.out, R.cfg, sa);
+            const size_t smem = SPEC_WARPS * (sizeof(avk_sp::Shared) + 32 * sizeof(avk_sp::Scratch));
+            if (R.out.strata) k_search_spec<true><<<sm, 32 * SPEC_WARPS, smem, strm>>>(R.db, R.out, R.cfg, sa);
+            else k_search_spec<false><<<sm, 32 * SPEC_WARPS, smem, strm>>>(R.db, R.out, R.cfg, sa);
             ctx->launches += 1;
             a.dense_blobs = sa.dense_blobs; a.dense_cap = dense_cap;
         }
@@ -1968,7 +2000,9 @@ static int run_compare_pipeline(avk_ctx *ctx, const CompareRun &R) {
         TierArgs a = tier_args(ctx, keys ? (const u32 *)ctx->fail_s.p : LW, 12, 19, LW2, 13, sizeof(avk_ts::Work), nullptr);
         a.batch_min = ctx->thread_batch_min;
         a.pop_budget = ctx->thread_pop_budget ? ctx->thread_pop_budget : (n >= 2500000 ? 64 : (n >= 1200000 ? 48 : 32));   // (the same with passes in flight: measured)
-        k_compare_thread<<<(unsigned)std::min<u64>((u64)sm, (n + THREAD_TPB - 1) / THREAD_TPB), THREAD_TPB, THREAD_TPB * sizeof(avk_ts::Work), ctx->side[0]>>>(R.db, R.out, R.cfg, a);
+        const unsigned ctas = (unsigned)std::min<u64>((u64)sm, (n + THREAD_TPB - 1) / THREAD_TPB);
+        if (R.out.strata) k_compare_thread<true><<<ctas, THREAD_TPB, THREAD_TPB * sizeof(avk_ts::Work), ctx->side[0]>>>(R.db, R.out, R.cfg, a);
+        else k_compare_thread<false><<<ctas, THREAD_TPB, THREAD_TPB * sizeof(avk_ts::Work), ctx->side[0]>>>(R.db, R.out, R.cfg, a);
         ctx->launches += 1;
         const int rc = spec_then_team(LW2, 13, 22, 23, ctx->dense_blobs2, (u8 *)ctx->arena2.p + spill_half, ctx->side[0]);   // W2 -> B
         if (rc != AVK_OK) return rc;
@@ -2032,23 +2066,16 @@ static int run_big_tiers(avk_ctx *ctx, const CompareRun &R, u32 n_work) {
     return AVK_OK;
 }
 
-// Summary counters: fold the partial tables (in-kernel totals), or -- when strata are requested -- reduce the per-region
-// rows (k_reduce also sums the strata).  Idempotent: may be run again after the cooperative tiers added their clusters.
+// Summary counters: fold the partial tables of the totals and, when strata are requested, of the per-stratum sums.
+// Idempotent: may be run again after the cooperative tiers added their clusters.
 static int run_finalize(avk_ctx *ctx, const CompareRun &R) {
-    const u64 n = ctx->n_regions;
-    unsigned long long *tot = (unsigned long long *)ctx->totals.p;
-    if (!R.strata) {
-        k_fold_slots<<<1, 320, 0, ctx->stream>>>((const unsigned long long *)ctx->tot_slots.p, tot);
+    k_fold_slots<<<1, 320, 0, ctx->stream>>>((const unsigned long long *)ctx->tot_slots.p, (unsigned long long *)ctx->totals.p);
+    ctx->launches += 1;
+    if (R.out.strata) {
+        const u64 cols = (u64)R.strata.n_strata * RED_COLS;
+        k_fold_strata<<<(unsigned)std::min<u64>((cols + 255) / 256, (u64)ctx->sm_count * 4), 256, 0, ctx->stream>>>(R.strata.slots, cols,
+                                                                                                                 (unsigned long long *)ctx->strat_totals.p);
         ctx->launches += 1;
-    } else {
-        CK(cudaMemsetAsync(tot, 0, 8 * RED_COLS + 64, ctx->stream));
-        CK(cudaMemsetAsync(ctx->strat_totals.p, 0, 8ull * RED_COLS * R.n_strata, ctx->stream));
-        if (n) {
-            k_reduce<<<(unsigned)std::min<u64>(n, (u64)ctx->sm_count * 8), 288, 0, ctx->stream>>>(
-                n, R.out.status, R.out.region_metrics, R.out.type_mask, tot, (u32 *)(tot + RED_COLS), tot + RED_COLS + 1, tot + RED_COLS + 2,
-                R.strat_off, R.strat_idx, R.strat_mask, (unsigned long long *)ctx->strat_totals.p);
-            ctx->launches += 1;
-        }
     }
     CK(cudaGetLastError());
     return AVK_OK;
@@ -2066,17 +2093,20 @@ static int queue_counter_copies(avk_ctx *ctx) {
 // Launches one compare pass over the resident batch; nothing waits for the device.
 static int compare_launch(avk_ctx *ctx, const avk_compare_cfg *cfg, bool want_seq, bool want_rows, bool strata, u32 n_strata, bool strat_dev, bool want_contain, CompareRun &R) {
     const u64 n = ctx->n_regions, nv = ctx->n_variants;
-    const bool rows = want_rows || strata;
     if (strat_dev || want_contain) ENSURE(ctx->st_mask, 8 * n);
     ENSURE(ctx->status, 4 * n); ENSURE(ctx->ed1, 4 * n); ENSURE(ctx->ed2, 4 * n);
-    if (rows) ENSURE(ctx->region_metrics, 8ull * RED_COLS * n);
+    if (want_rows) ENSURE(ctx->region_metrics, 8ull * RED_COLS * n);
     ENSURE(ctx->type_mask, 2 * n);
     ENSURE(ctx->vexp, nv); ENSURE(ctx->vobs, nv); ENSURE(ctx->vcls, nv);
     ENSURE(ctx->totals, 8 * RED_COLS + 64);
     ENSURE(ctx->tot_slots, 8ull * TOT_SLOTS * TOT_STRIDE);
     ENSURE(ctx->counters, 256);
     ENSURE(ctx->work_ctr, 64);
-    if (strata) ENSURE(ctx->strat_totals, 8ull * RED_COLS * n_strata);
+    if (strata) {
+        ENSURE(ctx->strat_totals, 8ull * RED_COLS * n_strata);
+        ENSURE(ctx->strat_slots, 8ull * STRAT_SLOTS * RED_COLS * n_strata);
+        CK(cudaMemsetAsync(ctx->strat_slots.p, 0, 8ull * STRAT_SLOTS * RED_COLS * n_strata, ctx->stream));
+    }
     CK(cudaMemsetAsync(ctx->work_ctr.p, 0, 64, ctx->stream));
     CK(cudaMemsetAsync(ctx->tot_slots.p, 0, 8ull * TOT_SLOTS * TOT_STRIDE, ctx->stream));
     // digest buffers are sized from a host-side upper bound, so no device round trip is needed
@@ -2086,19 +2116,28 @@ static int compare_launch(avk_ctx *ctx, const avk_compare_cfg *cfg, bool want_se
     R.db = dev_batch(ctx);
     DevCompareOut &out = R.out;
     out.status = (int *)ctx->status.p; out.ed1 = (u32 *)ctx->ed1.p; out.ed2 = (u32 *)ctx->ed2.p;
-    out.region_metrics = rows ? (u64 *)ctx->region_metrics.p : nullptr;
-    out.tot_slots = strata ? nullptr : (unsigned long long *)ctx->tot_slots.p;
+    out.region_metrics = want_rows ? (u64 *)ctx->region_metrics.p : nullptr;
+    out.tot_slots = (unsigned long long *)ctx->tot_slots.p;
     out.type_mask = (uint16_t *)ctx->type_mask.p;
     out.vexp = biased<u8>(ctx->vexp, ctx->v_base); out.vobs = biased<u8>(ctx->vobs, ctx->v_base); out.vcls = biased<u8>(ctx->vcls, ctx->v_base);
     out.seq_off = want_seq ? (const u64 *)ctx->seq_off.p : nullptr;
     out.seq_len = (u32 *)ctx->seq_len.p; out.seq_pool = biased<u8>(ctx->seq_pool, ctx->seq_base);
+    out.strata = nullptr;
+    if (strata) {
+        DevStrata &st = R.strata;
+        st.slots = (unsigned long long *)ctx->strat_slots.p;
+        st.n_strata = n_strata;
+        st.st_mask = strat_dev ? (const u64 *)ctx->st_mask.p : nullptr;
+        st.strat_off = strat_dev ? nullptr : (const u64 *)ctx->strat_off.p;
+        st.strat_idx = strat_dev ? nullptr : biased<const u32>(ctx->strat_idx, ctx->strat_base);
+        ENSURE(ctx->strat_args, sizeof(DevStrata));     // (on the pass's stream: ordered after the previous pass's kernels)
+        CK(cudaMemcpyAsync(ctx->strat_args.p, &st, sizeof(DevStrata), cudaMemcpyHostToDevice, ctx->stream));
+        out.strata = (const DevStrata *)ctx->strat_args.p;
+    }
     R.cfg = *cfg;
-    R.strata = strata; R.n_strata = n_strata;
-    R.strat_off = (strata && !strat_dev) ? (const u64 *)ctx->strat_off.p : nullptr;
-    R.strat_idx = (strata && !strat_dev) ? biased<const u32>(ctx->strat_idx, ctx->strat_base) : nullptr;
-    R.strat_mask = (strata && strat_dev) ? (const u64 *)ctx->st_mask.p : nullptr;
     R.want_contain = strat_dev || want_contain;
     ctx->have_result = ctx->have_merge = ctx->result_has_seq = false;
+    ctx->result_strata = 0;
 
     CK(cudaEventRecord(ctx->ev[0], ctx->stream));
     int rc = run_alt_ed(ctx, R.db);
@@ -2119,7 +2158,7 @@ static int compare_launch(avk_ctx *ctx, const avk_compare_cfg *cfg, bool want_se
     rc = run_finalize(ctx, R);
     if (rc != AVK_OK) return rc;
     CK(cudaEventRecord(ctx->ev[4], ctx->stream));
-    ctx->result_has_rows = rows;
+    ctx->result_has_rows = want_rows;
     ctx->result_has_seq = want_seq && cfg->enable_sequences;   // (the kernels emit the bundle only under enable_sequences)
     ctx->result_has_contain = R.want_contain;
     return queue_counter_copies(ctx);
@@ -2186,7 +2225,7 @@ static int download_compare_async(avk_ctx *ctx, avk_compare_out *out, bool want_
     const cudaStream_t ds = ctx->dn ? ctx->dn : ctx->stream;
     // st_mask holds whatever an earlier pass left there, possibly for a smaller batch
     if (out->containment && n && !ctx->result_has_contain) {
-        ctx->err = "containment masks were not computed by this run (avk_compare_run_resident never computes them)";
+        ctx->err = "containment masks were not computed by this run (avk_compare_run_resident computes them only with AVK_CMP_STRATA)";
         return AVK_ERR_INVALID;
     }
     if (ctx->dn) CK(cudaStreamWaitEvent(ctx->dn, ctx->ev_done, 0));
@@ -2250,7 +2289,7 @@ static int prepare_outputs_on_device(avk_ctx *ctx, const avk_compare_out *out, u
     strata = strata_wanted(out);
     strat_dev = strata && !out->strat_off;
     if ((strat_dev || out->containment) && (ref_of(ctx)->st_n == 0 || (strat_dev && ref_of(ctx)->st_n != out->n_strata) || ref_of(ctx)->st_contigs != (u32)ref_of(ctx)->contig_lens.size())) {
-        ctx->err = "the device containment lookup needs avk_set_stratifications (same number of strata as n_strata, contigs as the reference)";
+        ctx->err = DEVICE_LOOKUP_NEEDS;
         return AVK_ERR_INVALID;
     }
     if (strata && !strat_dev) {
@@ -2854,14 +2893,22 @@ extern "C" int avk_compare_run_resident(avk_ctx *ctx, const avk_compare_cfg *cfg
     if (!cfg || !ctx->have_batch || ctx->n_inputs != 2) { ctx->err = "no resident compare batch"; return AVK_ERR_INVALID; }
     const bool keep_seq = (cfg->flags & AVK_CMP_KEEP_SEQUENCES) != 0;
     if (keep_seq && !cfg->enable_sequences) { ctx->err = "AVK_CMP_KEEP_SEQUENCES needs enable_sequences"; return AVK_ERR_INVALID; }
+    const bool strata = (cfg->flags & AVK_CMP_STRATA) != 0;
+    const avk_ctx *so = ref_of(ctx);
+    if (strata && (so->st_n == 0 || so->st_contigs != (u32)so->contig_lens.size())) {
+        ctx->err = DEVICE_LOOKUP_NEEDS;
+        return AVK_ERR_INVALID;
+    }
+    const u32 n_strata = strata ? so->st_n : 0;
     CK(cudaSetDevice(ctx->device));
     CompareRun R;
     int rc = keep_seq ? resident_seq_layout(ctx) : AVK_OK;
     if (rc != AVK_OK) return rc;
-    rc = compare_launch(ctx, cfg, keep_seq, (cfg->flags & AVK_CMP_KEEP_REGION_ROWS) != 0, false, 0, false, false, R);
+    rc = compare_launch(ctx, cfg, keep_seq, (cfg->flags & AVK_CMP_KEEP_REGION_ROWS) != 0, strata, n_strata, strata, strata, R);
     if (rc != AVK_OK) return rc;
     rc = compare_finish(ctx, R, nullptr);
     if (rc != AVK_OK) return rc;
+    ctx->result_strata = n_strata;
     return fetch_timings(ctx);
 }
 
@@ -2869,15 +2916,20 @@ extern "C" int avk_compare_run_resident(avk_ctx *ctx, const avk_compare_cfg *cfg
 extern "C" int avk_compare_download(avk_ctx *ctx, avk_compare_out *out) {
     if (!ctx) return AVK_ERR_INVALID;
     if (!out || !ctx->have_batch || !ctx->have_result) { ctx->err = "no compare result is resident (run avk_compare_run_resident first)"; return AVK_ERR_INVALID; }
-    if (strata_wanted(out)) { ctx->err = "avk_compare_download returns no stratified sums: request them from avk_compare_batch*"; return AVK_ERR_INVALID; }
+    const bool strata = strata_wanted(out);
+    if (strata && (out->strat_off || !ctx->result_strata || out->n_strata != ctx->result_strata)) {
+        ctx->err = "avk_compare_download returns no stratified sums: only those of a resident run with AVK_CMP_STRATA, over its number of "
+                   "strata and without strat_off; request others from avk_compare_batch*";
+        return AVK_ERR_INVALID;
+    }
     CK(cudaSetDevice(ctx->device));
     int rc = download_compare_async(ctx, out, false, 0);
     if (rc != AVK_OK) return rc;
     CK(cudaStreamSynchronize(ctx->stream));
     BinTotals bt;
-    rc = collect_totals(ctx, out, false, bt);
+    rc = collect_totals(ctx, out, strata, bt);
     if (rc != AVK_OK) return rc;
-    store_totals(out, bt, false, false);
+    store_totals(out, bt, strata, false);
     return AVK_OK;
 }
 

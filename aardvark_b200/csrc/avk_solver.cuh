@@ -48,13 +48,34 @@ struct DevBatch {
 struct DevCompareOut {
     int *status;
     u32 *ed1, *ed2;
-    u64 *region_metrics;   // [n][13][22], or NULL when the caller wants neither per-region rows nor strata
-    unsigned long long *tot_slots;   // [TOT_SLOTS][TOT_STRIDE], or NULL (rows mode: k_reduce sums the rows instead)
+    u64 *region_metrics;   // [n][13][22], or NULL when the caller wants no per-region rows
+    unsigned long long *tot_slots;   // [TOT_SLOTS][TOT_STRIDE]
     uint16_t *type_mask;
     u8 *vexp, *vobs, *vcls;
     const u64 *seq_off;    // may be NULL
     u32 *seq_len;
     u8 *seq_pool;
+    const struct DevStrata *strata;   // per-stratum sums (device memory), or NULL when no strata are requested
+};
+
+// Per-stratum sums of a pass: partial tables [STRAT_SLOTS][n_strata][TOT_COLS].  Region r belongs to the strata of its
+// containment mask st_mask[r] (device lookup) when st_mask is set, else to strat_idx[strat_off[r] .. strat_off[r + 1]) (the
+// caller's list; strat_idx is biased so that the caller's offsets index it).  Kept behind one pointer in device memory so that
+// the solver kernels' parameter block (copied to the stack where its address is taken) does not grow.
+struct DevStrata {
+    unsigned long long *slots;
+    const u64 *st_mask;
+    const u64 *strat_off;
+    const u32 *strat_idx;
+    u32 n_strata;
+
+    // adds v to column `col` of every stratum region r belongs to, in this CTA's partial table (out of line: the solver
+    // kernels of a pass without strata keep their own code)
+    __device__ __noinline__ void add(u64 r, int col, unsigned long long v) const {
+        unsigned long long *t = slots + (size_t)(blockIdx.x & (STRAT_SLOTS - 1)) * n_strata * TOT_COLS + col;
+        if (st_mask) for (u64 m = st_mask[r]; m; m &= m - 1) atomicAdd(t + (size_t)(__ffsll((long long)m) - 1) * TOT_COLS, v);
+        else for (u64 s = strat_off[r], e = strat_off[r + 1]; s < e; ++s) atomicAdd(t + (size_t)strat_idx[s] * TOT_COLS, v);
+    }
 };
 
 struct DevMergeOut {
@@ -1538,7 +1559,9 @@ __device__ __noinline__ int RegionSolver<SMEM>::compare_score(u64 r, const avk_c
             const u64 v = LD64(gm + 8 * i);
             if (v) {
                 const int k = i / AVK_N_METRICS, m = i - k * AVK_N_METRICS;
-                atomicAdd(slot + (k == 0 ? 0 : (1 + slot_type[k - 1]) * AVK_N_METRICS) + m, (unsigned long long)v);
+                const int col = (k == 0 ? 0 : (1 + slot_type[k - 1]) * AVK_N_METRICS) + m;
+                atomicAdd(slot + col, (unsigned long long)v);
+                if (out.strata) out.strata->add(r, col, (unsigned long long)v);
             }
         }
         if (lane == 0) { atomicOr(slot + TOT_MASK, (unsigned long long)mask); atomicAdd(slot + TOT_SOLVED, 1ull); }

@@ -281,11 +281,14 @@ class Solver:
         else:
             self._check(self._lib.avk_compare_upload_range(self._ctx, C.byref(cb), lo, hi), "avk_compare_upload_range")
 
-    def run_resident(self, cfg: CompareConfig = None, region_metrics: bool = False, sequences: bool = False):
+    def run_resident(self, cfg: CompareConfig = None, region_metrics: bool = False, sequences: bool = False, strata: bool = False):
         """One pass over the resident batch.  region_metrics=True keeps the per-region metric rows on the device so
         that download() and writers.region_summary_bgzf can use them; sequences=True (needs cfg.enable_sequences) fills the
-        sequence bundle on the device for writers.region_sequences_bgzf (AVK_CMP_KEEP_SEQUENCES; a slower pass)."""
-        flags = (abi.CMP_KEEP_REGION_ROWS if region_metrics else 0) | (abi.CMP_KEEP_SEQUENCES if sequences else 0)
+        sequence bundle on the device for writers.region_sequences_bgzf (AVK_CMP_KEEP_SEQUENCES; a slower pass);
+        strata=True computes the containment masks and per-stratum sums through the tables of set_stratifications
+        (AVK_CMP_STRATA) for resident_sums() and download()."""
+        flags = ((abi.CMP_KEEP_REGION_ROWS if region_metrics else 0) | (abi.CMP_KEEP_SEQUENCES if sequences else 0) |
+                 (abi.CMP_STRATA if strata else 0))
         cc = compare_cfg(cfg or CompareConfig(enable_sequences=False), flags)
         self._check(self._lib.avk_compare_run_resident(self._ctx, C.byref(cc)), "avk_compare_run_resident")
 
@@ -298,6 +301,22 @@ class Solver:
         co = out.to_c()
         self._check(self._lib.avk_compare_download(self._ctx, C.byref(co)), "avk_compare_download")
         return out
+
+    def resident_sums(self, n_strata: int = 0):
+        """The summary counters of the resident bin's last pass without its batch on the host: (totals [13][22],
+        strat_totals [n_strata][13][22] or None, solved blocks, error blocks).  n_strata > 0 needs a pass with
+        run_resident(strata=True) over that many strata.  totals / strat_totals go to SummaryWriter.summary_text as they are;
+        the sums of several bins or lanes add up."""
+        v = self.result_device_view()
+        status = np.zeros(max(int(v.lo + v.n_regions), 1), dtype=np.int32)    # (the one array avk_compare_download requires)
+        totals = np.zeros((abi.N_GROUPS, abi.N_METRICS), dtype=np.uint64)
+        strat = np.zeros((n_strata, abi.N_GROUPS, abi.N_METRICS), dtype=np.uint64) if n_strata else None
+        solved, errors = np.zeros(1, dtype=np.uint64), np.zeros(1, dtype=np.uint64)
+        co = abi.CompareOut()
+        co.status, co.totals, co.solved_blocks, co.error_blocks = abi.ptr(status), abi.ptr(totals), abi.ptr(solved), abi.ptr(errors)
+        co.n_strata, co.strat_totals = int(n_strata), abi.ptr(strat)
+        self._check(self._lib.avk_compare_download(self._ctx, C.byref(co)), "avk_compare_download")
+        return totals, strat, int(solved[0]), int(errors[0])
 
     # -- resident merge: upload (or build_regions), solve, and write the outputs where the batch lies -------------------
     def merge_upload(self, batch: RegionBatch, lo: int = None, hi: int = None):

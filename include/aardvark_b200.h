@@ -182,6 +182,13 @@ typedef struct avk_compare_cfg {
  * there instead: measured on a B200, the chr20-shaped pass (115 k clusters) takes 6.9 ms with the bundle against 3.3 ms with
  * the rows only.  avk_compare_batch* decide from the out->seq_* pointers. */
 #define AVK_CMP_KEEP_SEQUENCES 2u
+/* avk_compare_run_resident: a stratified pass.  The containment masks of the resident bin are computed through the
+ * stratification tables (avk_set_stratifications; a lane reads its owner's) and the solver stages add every solved cluster's
+ * metrics to the sums of its strata, so that avk_compare_download can return out->containment and out->strat_totals without
+ * the batch or per-region rows on the host.  Refused (AVK_ERR_INVALID, the context stays usable) when no tables are set or
+ * when they were built for a reference with another number of contigs.  Combines with the two flags above; without it the
+ * pass is the plain one. */
+#define AVK_CMP_STRATA 4u
 
 /* MergeConfig, src/merge_solver.rs:62-84 */
 typedef struct avk_merge_cfg {
@@ -529,9 +536,12 @@ int avk_merge_summary_rows_write(const avk_merge_summary_row *rows, uint64_t n_r
 int avk_compare_upload(avk_ctx *ctx, const avk_region_batch *batch);
 int avk_compare_upload_range(avk_ctx *ctx, const avk_region_batch *batch, uint64_t lo, uint64_t hi);
 int avk_compare_run_resident(avk_ctx *ctx, const avk_compare_cfg *cfg);
-/* copies the resident bin's results into out->...[lo..hi) / [v_base..) of the caller's arrays.  AVK_ERR_INVALID when out
- * asks for what the last pass did not compute: region_metrics after a run without AVK_CMP_KEEP_REGION_ROWS, containment
- * after avk_compare_run_resident (which never computes it), and stratified sums (strat_totals with n_strata > 0) always:
+/* copies the resident bin's results into out->...[lo..hi) / [v_base..) of the caller's arrays; only out->status is required.
+ * After a resident run with AVK_CMP_STRATA it also fills out->containment and out->strat_totals (this bin's sums; add them
+ * up over bins or lanes) when out->strat_off is NULL and out->n_strata is the number of strata that run used (kept with
+ * the result: tables replaced since do not change it).  AVK_ERR_INVALID when out asks for what the last pass did not
+ * compute: region_metrics after a run without AVK_CMP_KEEP_REGION_ROWS, containment after a resident run without
+ * AVK_CMP_STRATA, and stratified sums in every other case (a membership list, another n_strata, a run without the flag):
  * request those from avk_compare_batch*. */
 int avk_compare_download(avk_ctx *ctx, avk_compare_out *out);
 /* DEVICE addresses of the resident bin's results (valid until the next call on the context): what a
